@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MSACL fused rollout hot path (BASELINE.json metric: fused env-steps/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--env NAME] [--envs-per-gpu M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--env NAME] [--envs-per-gpu M] [--dump-outputs DIR]
 
 Headline workload (config 5 of BASELINE.json, per-GPU share): QuadTracking, 2^21 env instances per GPU
 (16 Mi envs on 8 GPUs), default-init StochaPolicy actor (seed 0), Philox resets, one "step" =
@@ -356,6 +356,22 @@ def time_rollout(cx, env, n, K, engine, steps, warmup, keep=False, clocks=False,
     return out
 
 
+def last_launch_outputs(ro, env_base, seed=0, budget=48 << 20):
+    """What the last launch of `ro` handed its caller: the K new transition slices ([K, m, .] per field, float32), for
+    all n env instances or, beyond `budget` bytes, a fixed seeded sample of m of them; `env_index` holds the global
+    env ids of the m columns."""
+    import torch
+    tr = ro.tr
+    fields = {k: v[tr.H:] for k, v in tr.fields().items()}
+    per_env = 4 * sum(v[:, 0].numel() for v in fields.values())
+    m = min(tr.n, max(1, budget // per_env))
+    idx = np.arange(tr.n) if m == tr.n else np.sort(np.random.default_rng(seed).choice(tr.n, m, replace=False))
+    cols = torch.as_tensor(idx, device=fields["obs"].device)
+    out = {k: v.index_select(1, cols).float().cpu().numpy() for k, v in fields.items()}
+    out["env_index"] = (idx + env_base).astype(np.float64)
+    return out
+
+
 def time_general_rollout(cx, env="TwoLink", n=1 << 18, K=16, hidden=(64, 64), steps=3, warmup=2):
     """The general rollout engine (a policy the fused kernels are not specialised for: per-layer tcgen05 GEMMs +
     msacl_rollout_step, launches per env step instead of one per K steps)."""
@@ -560,8 +576,10 @@ def time_training_loop(cx, env="VanderPol", iters=60):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed launches of the headline rollout, of the e2e region and of every rollout in `configs`; the "
+                         "target-kernel, learner and training-loop configs time fixed repetition counts of their own")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed launches before each timed region (at least 3 for b200)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--env", default="QuadTracking")
     ap.add_argument("--envs-per-gpu", type=int, default=1 << 21)
@@ -583,7 +601,15 @@ def main():
     ap.add_argument("--reserve-sms", type=int, default=0, help="N>1 e2e: SMs left free for the side-stream NCCL all-gather")
     ap.add_argument("--replay", default="indexed", choices=["indexed", "ring"],
                     help="e2e replay store: index-based windows over the transition store (default) or the reference-layout ring")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the transitions of the last timed launch (rank 0; a fixed seeded sample of about 48 MB of env "
+                         "instances when all of them are more) as DIR/<field>.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the b200 rollout")
+    if args.dump_outputs and args.settle > 0:
+        ap.error("--dump-outputs needs --settle 0: the number of settling launches, and so the state the timed launches "
+                 "start from, depends on timing")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -649,6 +675,10 @@ def main():
     ro, host_w = main_run["ro"], main_run["host_w"]
     value, total_ms, kern_ms, clk = main_run["value"], main_run["total_ms"], main_run["kern_ms"], main_run["clocks"]
     main_run_burst = main_run["value_burst"]
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in last_launch_outputs(ro, rank * n).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     steps_total = n * K * args.steps * world
     h2d_bytes = sum(p.numel() * 4 for p in host_w)
 
@@ -780,7 +810,7 @@ def main():
     configs = None
     if not args.no_configs:
         configs = {}
-        S, W = max(3, min(args.steps, 5)), 3
+        S, W = args.steps, args.warmup
 
         def rollout_cfg(env, n_c, K_c, engine="tc"):
             r = time_rollout(cx, env, n_c, K_c, engine, S, W)
@@ -804,7 +834,7 @@ def main():
             configs["3_twolink_1M_envs_msacl_targets"] = c3
             configs["5_quadtracking_fp32_ffma_engine"] = rollout_cfg(args.env, n, K, "ffma" if args.engine == "tc" else "tc")
             try:
-                configs["general_engine_twolink_hidden_64x64_tanh"] = time_general_rollout(cx)
+                configs["general_engine_twolink_hidden_64x64_tanh"] = time_general_rollout(cx, steps=S, warmup=W)
             except Exception as e:
                 configs["general_engine_twolink_hidden_64x64_tanh"] = {"error": repr(e)}
             try:

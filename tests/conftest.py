@@ -8,6 +8,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+sys.path.insert(0, GOLDEN)
+from golden_params import unpack_parameters  # noqa: E402
 
 
 def pytest_configure(config):
@@ -15,7 +17,10 @@ def pytest_configure(config):
 
 
 def load_golden(name):
-    return dict(np.load(os.path.join(GOLDEN, name), allow_pickle=False))
+    g = dict(np.load(os.path.join(GOLDEN, name), allow_pickle=False))
+    if "init_seed" in g:            # network parameters stored compactly (golden_params.py); restoring them needs torch
+        unpack_parameters(g)
+    return g
 
 
 @pytest.fixture(scope="session")

@@ -10,6 +10,7 @@ Shims (SURVEY.md section 8c): a gymnasium 0.28.1 stub (tests/golden/_gym_stub), 
 host (RL/algorithm/msacl.py:156-164 call .cuda() unconditionally).  The reference sources are
 not modified; attribute overrides on *instances* (env.max_step, env.obs, ...) only set state.
 """
+import json
 import os
 import random
 import sys
@@ -27,6 +28,8 @@ torch.Tensor.cuda = lambda self, *a, **k: self
 torch.nn.Module.cuda = lambda self, *a, **k: self
 
 from RL.env.make_env import make_env  # noqa: E402
+
+from golden_params import msacl_init_params, pack_parameters  # noqa: E402
 
 f32 = np.float32
 ENVS = ["VanderPol", "Pendulum", "DuctedFan", "TwoLink", "SingleTrackCar", "QuadTracking"]
@@ -456,12 +459,41 @@ def extra_cases():
         print("wrote", path, {k: data[k] for k in ("trm", "trs", "tcm", "tcs")}, data["first_episode_len"])
 
 
+def packed_targets_case(seed=11):
+    out = msacl_case(seed=seed)
+    names = [str(n) for n in out["lya_param_names"]]
+    return pack_parameters(out, seed, out["obs"].shape[-1], out["act"].shape[-1], ["lya_param_" + n for n in names],
+                           ["lyapunov." + n for n in names], [], [])
+
+
+def packed_update_case(seed=21):
+    out = msacl_update_case(seed=seed)
+    D, A = out["data_obs"].shape[-1], out["data_act"].shape[-1]
+    keys = [str(k) for k in out["state_keys"]]
+    init = [k for k in keys if k in msacl_init_params(seed, D, A)]
+    return pack_parameters(out, seed, D, A, ["before_" + k for k in init], init, ["after_" + k for k in keys],
+                           ["before_" + k for k in keys])
+
+
+def tb_tags_case():
+    """The reference's TensorBoard tag table (RL/utils/tensorboard_setup.py:13-40): a naming contract with its CSV /
+    plotting tools that msacl_b200.trainer.tb_tags keeps."""
+    from RL.utils.tensorboard_setup import tb_tags
+    path = os.path.join(HERE, "reference_tb_tags.json")
+    with open(path, "w") as fh:
+        json.dump(tb_tags, fh, indent=1)
+        fh.write("\n")
+    print("wrote", path)
+
+
 def main():
     if "--only-extra" in sys.argv:
         return extra_cases()
+    if "--only-tags" in sys.argv:
+        return tb_tags_case()
     if "--only-update" in sys.argv:
         path = os.path.join(HERE, "msacl_update_TwoLink.npz")
-        np.savez_compressed(path, **msacl_update_case())
+        np.savez_compressed(path, **packed_update_case())
         print("wrote", path)
         return
     rng = np.random.default_rng(20261018)
@@ -476,12 +508,13 @@ def main():
         np.savez_compressed(path, **data)
         print("wrote", path, "windows:", len(data["win_rew"]), "dones:", int(data["step_done"].sum()))
     path = os.path.join(HERE, "msacl_targets_TwoLink.npz")
-    np.savez_compressed(path, **msacl_case())
+    np.savez_compressed(path, **packed_targets_case())
     print("wrote", path)
     path = os.path.join(HERE, "msacl_update_TwoLink.npz")
-    np.savez_compressed(path, **msacl_update_case())
+    np.savez_compressed(path, **packed_update_case())
     print("wrote", path)
     extra_cases()
+    tb_tags_case()
 
 
 if __name__ == "__main__":
