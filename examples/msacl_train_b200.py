@@ -5,6 +5,9 @@
 `env_num` is raised (the GPU steps thousands of envs per launch) and logging is plain stdout.
 
     python examples/msacl_train_b200.py --env_name VanderPol --max_iteration 2000
+
+With --certify_states N the trained controller's Lyapunov certificate is then checked on N initial states (msacl_b200.
+create_certifier; an empirical check over the sampled states and n_step steps, not a proof) and the report printed as JSON.
 """
 import argparse
 import os
@@ -34,6 +37,8 @@ def main():
     p.add_argument("--num_eval_episode", type=int, default=64)
     p.add_argument("--rollout_engine", default="tc")
     p.add_argument("--seed", type=int, default=0)
+    p.add_argument("--certify_states", type=int, default=0, help="after training, check the Lyapunov certificate on this many "
+                   "initial states (0: skip)")
     a = vars(p.parse_args())
     spec = get_spec(a["env_name"])
     torch.manual_seed(a["seed"])
@@ -60,6 +65,11 @@ def main():
             env_steps = sampler.get_total_sample_number()
             print(f"iter {it:6d}  env-steps {env_steps:10d}  TRM {trm:10.3f} +- {trs:8.3f}  TCM {tcm:10.4f} +- {tcs:8.4f}  "
                   f"loss_q {info['Loss/Critic loss-RL iter'] if info else float('nan'):10.3f}  wall {time.time() - t0:6.1f}s", flush=True)
+    if a["certify_states"] > 0:
+        report = msacl_b200.create_certifier(networks=alg.networks, env_name=a["env_name"], num_states=a["certify_states"],
+                                             horizon=a["n_step"], lya_eta=kw["lya_eta"], alpha1=kw["alpha1"], alpha2=kw["alpha2"],
+                                             seed=a["seed"], rollout_engine=a["rollout_engine"]).run()
+        print("certificate", report.to_json(), flush=True)
 
 
 if __name__ == "__main__":

@@ -396,6 +396,78 @@ int msacl_selftest_tc_gemm(const float* A, const float* W, float* D, int32_t spl
  * mbarrier wait per group.  cycles_per_umma: device double[4]. */
 int msacl_umma_probe(int32_t mode, int32_t iters, double* cycles_per_umma, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Lyapunov-certificate verifier (no counterpart in the reference).  For every initial state i the caller runs the greedy
+ * closed loop for up to `horizon` steps (msacl_rollout_fused* with deterministic = 1, n_step = 1, max_step > horizon) and
+ * evaluates V = networks.lyapunov on the visited observations; these entry points check, per visited state k = 0..e
+ * (e = the first step whose `done` is set, else horizon), with s_k = sum_j o_k[j]^2 accumulated in float64 in order j = 0..D-1,
+ * c_k = decay[k] and every comparison in float64:
+ *   NONFINITE       some o_k[j] or V_k is NaN / Inf
+ *   BOUND_LO        V_k < alpha1 s_k - v_atol              BOUND_HI  V_k > alpha2 s_k + v_atol
+ *   DECREASE        k >= 1 and V_k > c_k V_0 + v_atol       ESCAPED   done at some step k <= horizon
+ *   NOT_EXP_STABLE  k >= 1 and s_k > (alpha2 / alpha1) c_k s_0   (model-free; independent of V)
+ * A state is certified when it has none of the first five.  An empirical check over the sampled states and horizon, not
+ * a proof.  Records are per state, structure-of-arrays, streamed chunk by chunk: memory is O(n), not O(n * horizon).
+ * --------------------------------------------------------------------------------------------------------------- */
+enum {
+  MSACL_CERT_NONFINITE = 1,
+  MSACL_CERT_BOUND_LO = 2,
+  MSACL_CERT_BOUND_HI = 4,
+  MSACL_CERT_DECREASE = 8,
+  MSACL_CERT_ESCAPED = 16,
+  MSACL_CERT_NOT_EXP_STABLE = 32,
+  MSACL_CERT_FAIL_MASK = 31,          /* flags that make a state uncertified */
+  MSACL_CERT_MAX_HORIZON = 8192
+};
+
+/* Layout of the int64 summary written by msacl_certify_finish / msacl_certify_roa: [MSACL_CERT_SUM_HIST + horizon] */
+enum {
+  MSACL_CERT_SUM_STATES = 0,          /* n */
+  MSACL_CERT_SUM_FLAGS = 1,           /* [1 + b] = states with flag bit b set, b = 0..5 */
+  MSACL_CERT_SUM_CERTIFIED = 7,
+  MSACL_CERT_SUM_INCONSISTENT = 8,    /* states where DECREASE and NOT_EXP_STABLE disagree */
+  MSACL_CERT_SUM_CSTAR_KEY = 9,       /* min V_0 over uncertified states with V_0 not NaN, as the order-preserving key of its
+                                         float32 bits (bits | 0x80000000 for sign 0, ~bits for sign 1); +inf if none */
+  MSACL_CERT_SUM_ROA = 10,            /* #{i : V_0,i < c_star} (msacl_certify_roa) */
+  MSACL_CERT_SUM_HIST = 11            /* [11 + k - 1] = states whose first DECREASE is at step k, k = 1..horizon */
+};
+
+typedef struct {
+  int32_t horizon;         /* T, 1..MSACL_CERT_MAX_HORIZON; steps k > T are ignored */
+  double alpha1, alpha2;   /* > 0 */
+  double v_atol;           /* >= 0, absolute slack on V */
+  const double* decay;     /* device double[T + 1]: c_0 = 1, c_k = c_{k-1} (1 - eta) (repeated multiplication) */
+} msacl_cert_params_t;
+
+/* Per-state records, device arrays [n] */
+typedef struct {
+  float* v0;               /* V(o_0) */
+  double* s0;              /* s_0 */
+  uint8_t* flags;          /* MSACL_CERT_* bits */
+  int32_t* first_violation;/* first k at which a flag of MSACL_CERT_FAIL_MASK was raised, -1 if none */
+  int32_t* first_decrease; /* first k with DECREASE, -1 if none */
+  int32_t* end_step;       /* e */
+  double* worst_ratio;     /* max_{1<=k<=e} V_k / (c_k V_0); 0/0 = 0, x/0 = +inf for x > 0, NaN terms skipped; 0 if e = 0 */
+} msacl_cert_records_t;
+
+/* Box initial states: o_i[j] = lo[j] + (hi[j] - lo[j]) u (float32), u = top 24 bits of Philox4x32-10 word 0 for the counter
+ * (env_base + i, j, 0x63657274) under key st->seed, written into the sf rows of the five box envs (state == observation).
+ * lo / hi: HOST float[obs_dim], lo <= hi.  Call after msacl_env_reset (which zeroes the step counters). */
+int msacl_certify_box_init(const msacl_env_state_t* st, const float* lo, const float* hi, void* stream);
+/* Initialise the records from the initial observations obs0 [n][obs_dim] and v0 [n] (checks of k = 0). */
+int msacl_certify_begin(int64_t n, int32_t obs_dim, const float* obs0, const float* v0, const msacl_cert_params_t* p,
+                        const msacl_cert_records_t* rec, void* stream);
+/* One rollout chunk of K steps k0 .. k0 + K - 1 (k0 >= 1) in the transition-store layout: obs2 [K][n][obs_dim] (the real
+ * next observation), v [K][n] = V(obs2), done [K][n].  States that already ended are skipped; obs2 rows are read with
+ * 16-byte (obs_dim % 4 == 0) or 8-byte (even) vector loads and must be aligned accordingly. */
+int msacl_certify_steps(int64_t n, int32_t obs_dim, int32_t K, int32_t k0, const float* obs2, const float* v, const uint8_t* done,
+                        const msacl_cert_params_t* p, const msacl_cert_records_t* rec, void* stream);
+/* Reduce the records into summary (zeroed by the call except [MSACL_CERT_SUM_ROA]): counts, first-DECREASE histogram and
+ * the c_star key.  One atomic per block and counter. */
+int msacl_certify_finish(int64_t n, int32_t horizon, const msacl_cert_records_t* rec, int64_t* summary, void* stream);
+/* summary[MSACL_CERT_SUM_ROA] = #{i < n : v0[i] < c_star} (zeroed by the call). */
+int msacl_certify_roa(int64_t n, const float* v0, float c_star, int64_t* summary, void* stream);
+
 const char* msacl_last_error(void);
 int msacl_abi_version(void);
 

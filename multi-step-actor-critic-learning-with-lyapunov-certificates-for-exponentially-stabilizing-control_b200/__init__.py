@@ -6,7 +6,7 @@ upstream project; `msacl_b200.py` at the repo root aliases it).
 from .specs import ENV_NAMES, SPECS, get_spec  # noqa: F401
 
 __all__ = ["ENV_NAMES", "SPECS", "get_spec", "create_envs", "create_sampler", "create_buffer", "create_alg", "create_evaluator",
-           "create_trainer", "load_library"]
+           "create_trainer", "create_certifier", "load_library"]
 
 
 def load_library():
@@ -64,3 +64,11 @@ def create_trainer(alg, sampler, buffer, evaluator, **kwargs):
     if name not in ("nstep_off_serial_trainer", "b200_nstep_off_serial_trainer"):
         raise KeyError(f"No registered trainer with id: {name}")
     return B200NstepOffSerialTrainer(alg, sampler, buffer, evaluator, **kwargs)
+
+
+def create_certifier(**kwargs):
+    """Lyapunov-certificate verifier of a trained ApproxContainer (no counterpart in the reference): closed-loop checks of
+    alpha1 |o|^2 <= V(o) <= alpha2 |o|^2 and of V's (1 - eta)^k decrease over many initial states -- an empirical check over
+    the sampled states and horizon, not a proof.  `create_certifier(networks=..., env_name=..., num_states=N).run()`."""
+    from .certify import B200CertificateVerifier
+    return B200CertificateVerifier(**kwargs)

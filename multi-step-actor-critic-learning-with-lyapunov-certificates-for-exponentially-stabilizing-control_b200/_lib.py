@@ -49,6 +49,15 @@ class Gemm(C.Structure):
                 ("row_sumsq", vp), ("precision", C.c_int32), ("b_packed", vp)]
 
 
+class CertParams(C.Structure):
+    _fields_ = [("horizon", C.c_int32), ("alpha1", C.c_double), ("alpha2", C.c_double), ("v_atol", C.c_double), ("decay", vp)]
+
+
+class CertRecords(C.Structure):
+    _fields_ = [("v0", vp), ("s0", vp), ("flags", vp), ("first_violation", vp), ("first_decrease", vp), ("end_step", vp),
+                ("worst_ratio", vp)]
+
+
 f32 = C.c_float
 i32, i64 = C.c_int32, C.c_int64
 
@@ -108,6 +117,11 @@ SIGNATURES = {
     "msacl_adam_tick": (C.c_int, [vp, vp, C.c_double, C.c_double, C.c_double, vp]),
     "msacl_ffma_probe": (C.c_int, [C.c_int32, C.c_int32, vp, c_f64p, vp]),
     "msacl_umma_probe": (C.c_int, [C.c_int32, C.c_int32, vp, vp]),
+    "msacl_certify_box_init": (C.c_int, [C.POINTER(EnvState), c_f32p, c_f32p, vp]),
+    "msacl_certify_begin": (C.c_int, [i64, i32, vp, vp, C.POINTER(CertParams), C.POINTER(CertRecords), vp]),
+    "msacl_certify_steps": (C.c_int, [i64, i32, i32, i32, vp, vp, vp, C.POINTER(CertParams), C.POINTER(CertRecords), vp]),
+    "msacl_certify_finish": (C.c_int, [i64, i32, C.POINTER(CertRecords), vp, vp]),
+    "msacl_certify_roa": (C.c_int, [i64, vp, f32, vp, vp]),
 }
 
 

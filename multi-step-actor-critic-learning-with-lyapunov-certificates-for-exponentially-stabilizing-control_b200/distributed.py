@@ -4,6 +4,8 @@ number of GPUs).  Collectives (NCCL on GPUs, gloo in the CPU tests) are used onl
 per-chunk episode statistics and for assembling a global replay batch from per-rank
 sub-batches (SURVEY.md section 8e).
 """
+import struct
+
 import torch
 import torch.distributed as dist
 
@@ -197,3 +199,42 @@ def episode_summary(stats):
     ep = max(s[0], 1.0)
     return {"episodes": int(s[0]), "mean_return": s[1] / ep, "mean_length": s[2] / ep, "terminated": int(s[3]),
             "truncated": int(s[4])}
+
+
+def float_order_key(x):
+    """Order-preserving uint32 key of a float32 (as the certificate verifier's atomicMin uses): bits | 0x80000000 for sign 0,
+    ~bits for sign 1.  Returns a Python int."""
+    b = struct.unpack("<I", struct.pack("<f", float(x)))[0]
+    return (~b & 0xFFFFFFFF) if b & 0x80000000 else (b | 0x80000000)
+
+
+def float_from_order_key(key):
+    """Inverse of `float_order_key`."""
+    key = int(key) & 0xFFFFFFFF
+    b = (key & 0x7FFFFFFF) if key & 0x80000000 else (~key & 0xFFFFFFFF)
+    return struct.unpack("<f", struct.pack("<I", b))[0]
+
+
+CERT_CSTAR_KEY, CERT_ROA = 9, 10        # MSACL_CERT_SUM_CSTAR_KEY / MSACL_CERT_SUM_ROA of include/msacl_b200.h
+
+
+def combine_certificate(summary, count_below):
+    """Combine the per-rank certificate summaries (int64 [11 + horizon], layout MSACL_CERT_SUM_* of include/msacl_b200.h) of
+    states sharded over ranks: counters and histogram are summed, the c_star key is all-reduced with MIN, and then
+    `count_below(c_star)` -- this rank's #{i : V_0,i < c_star} -- is summed into the ROA slot.  Returns (summary, c_star) with
+    the same values on every rank; single process: the local summary with its own c_star."""
+    s = summary.detach().to(torch.int64).clone()
+    key = s[CERT_CSTAR_KEY:CERT_CSTAR_KEY + 1].clone()
+    s[CERT_CSTAR_KEY] = 0
+    s[CERT_ROA] = 0
+    sharded = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+    if sharded:
+        dist.all_reduce(s, op=dist.ReduceOp.SUM)
+        dist.all_reduce(key, op=dist.ReduceOp.MIN)
+    c_star = float_from_order_key(int(key.item()))
+    roa = torch.tensor([int(count_below(c_star))], dtype=torch.int64, device=s.device)
+    if sharded:
+        dist.all_reduce(roa, op=dist.ReduceOp.SUM)
+    s[CERT_CSTAR_KEY] = key[0]
+    s[CERT_ROA] = roa[0]
+    return s, c_star

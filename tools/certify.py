@@ -1,0 +1,59 @@
+#!/usr/bin/env python
+"""Check the Lyapunov certificate of a trained checkpoint on the GPU and print the report as one JSON line.
+
+    python tools/certify.py --env_name VanderPol --checkpoint runs/apprfunc/apprfunc_2000.pkl --num_states 1048576
+
+The checkpoint is the trainer's `apprfunc_{iteration}.pkl` (`networks.state_dict()`); it is loaded into an ApproxContainer
+built with the network arguments of examples/msacl_train_b200.py (reference defaults, lyapunov_output_dim 256; override
+with the flags below).  The result is an empirical check over the sampled initial states and the horizon, not a proof.
+"""
+import argparse
+import json
+import os
+import sys
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+
+import torch  # noqa: E402
+
+import msacl_b200  # noqa: E402
+from msacl_b200.algorithm import ApproxContainer  # noqa: E402
+from msacl_b200.specs import get_spec  # noqa: E402
+
+
+def network_kwargs(env_name, lyapunov_output_dim=256):
+    """The ApproxContainer arguments of examples/msacl_train_b200.py (learning rates only size the unused optimisers)."""
+    spec = get_spec(env_name)
+    return dict(obs_dim=spec.obs_dim, act_dim=spec.act_dim, action_low_limit=spec.act_low, action_high_limit=spec.act_high,
+                lyapunov_output_dim=lyapunov_output_dim, q_learning_rate=1e-3, lyapunov_learning_rate=1e-3,
+                policy_learning_rate=3e-4, alpha_learning_rate=1e-3)
+
+
+def main(argv=None):
+    p = argparse.ArgumentParser()
+    p.add_argument("--env_name", default="VanderPol")
+    p.add_argument("--checkpoint", required=True, help="apprfunc_{iteration}.pkl written by the trainer")
+    p.add_argument("--num_states", type=int, default=1 << 20)
+    p.add_argument("--horizon", type=int, default=20, help="closed-loop steps per initial state (default: n_step = 20)")
+    p.add_argument("--lya_eta", type=float, default=0.15)
+    p.add_argument("--alpha1", type=float, default=1.0)
+    p.add_argument("--alpha2", type=float, default=2.0)
+    p.add_argument("--v_atol", type=float, default=0.0)
+    p.add_argument("--seed", type=int, default=0)
+    p.add_argument("--box", type=float, nargs=2, metavar=("LO", "HI"), help="uniform initial states in [LO, HI]^obs_dim "
+                   "(box envs) instead of the env's reset distribution")
+    p.add_argument("--lyapunov_output_dim", type=int, default=256)
+    p.add_argument("--rollout_engine", default="tc")
+    a = p.parse_args(argv)
+    nets = ApproxContainer(**network_kwargs(a.env_name, a.lyapunov_output_dim)).cuda()
+    nets.load_state_dict(torch.load(a.checkpoint, map_location="cuda", weights_only=True))
+    ver = msacl_b200.create_certifier(networks=nets, env_name=a.env_name, num_states=a.num_states, horizon=a.horizon,
+                                      lya_eta=a.lya_eta, alpha1=a.alpha1, alpha2=a.alpha2, v_atol=a.v_atol, seed=a.seed,
+                                      init=("box", a.box[0], a.box[1]) if a.box else "reset", rollout_engine=a.rollout_engine)
+    rep = ver.run()
+    print(rep.to_json(), flush=True)
+    return json.loads(rep.to_json())
+
+
+if __name__ == "__main__":
+    main()
