@@ -139,9 +139,7 @@ int msacl_rollout_fused(const msacl_env_state_t* st, const msacl_actor_t* actor,
  * in TMEM; layer 3, sampling and the dynamics stay FP32.  Logits agree with the FP32 path to ~3e-5
  * relative (tolerances in tests/test_gpu_tc.py).  w1p / w2p are the operand images produced by
  * msacl_tc_pack_actor (sizes from msacl_tc_pack_bytes); repack after every weight update.  The w2p buffer is the
- * 256 KB W2 image, followed -- only in builds with MSACL_TC_TPW=2 (two tiles per env warpgroup, experimental) -- by the
- * rollout kernel's per-CTA scratch area (logits hand-over of the tiles in flight), which msacl_rollout_fused_tc WRITES:
- * in such builds a given w2p buffer may be used by one launch at a time. */
+ * 256 KB W2 image; msacl_rollout_fused_tc only reads it. */
 int msacl_tc_pack_bytes(int64_t* w1p_bytes, int64_t* w2p_bytes);
 /* Process-wide grid cap of the persistent tensor-core rollout kernel: 0 (default) = one CTA per SM (148); a smaller value
  * leaves SMs free for a kernel that must run CONCURRENTLY with a rollout launch -- e.g. the NCCL all-gather of the replay

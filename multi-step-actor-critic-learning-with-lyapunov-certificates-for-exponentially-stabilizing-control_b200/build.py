@@ -30,10 +30,7 @@ NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",
     "-fmad=false",            # dynamics must round like NumPy scalar math; GEMMs call __fmaf_rn explicitly
     "-Xcompiler", "-fPIC", "-Xcompiler", "-ffp-contract=off",
-] + (["-DMSACL_TC_NS(ID)=" + os.environ["MSACL_TC_NS"]] if os.environ.get("MSACL_TC_NS") else []) \
-  + (["-DMSACL_TC_TPW(ID)=" + os.environ["MSACL_TC_TPW"]] if os.environ.get("MSACL_TC_TPW") else []) \
-  + os.environ.get("MSACL_NVCC_EXTRA", "").split() \
-  + (["-DMSACL_TC_TIMING"] if os.environ.get("MSACL_TC_TIMING") else []) \
+] + (["-DMSACL_TC_TIMING"] if os.environ.get("MSACL_TC_TIMING") else []) \
   + (["-DMSACL_TC_WATCHDOG"] if os.environ.get("MSACL_TC_WATCHDOG") else [])   # role timers / watchdog: tools/tc_*.py
 
 

@@ -202,13 +202,6 @@ template <> struct Env<kTwoLink> {
       const double b1 = ((double)a[0] - Cq1) - (double)G1;
       const double b2 = ((double)a[1] - Cq2) - (double)G2;
       const double m11 = (double)M11, m12 = (double)M12;
-#ifdef MSACL_TWOLINK_LU
-      const double l21 = m12 / m11;
-      const double u22 = M22 - l21 * m12;
-      const double y2 = b2 - l21 * b1;
-      const double x2 = y2 / u22;
-      const double x1 = (b1 - m12 * x2) / m11;
-#else
       // The LU solve above written out: x2 = (m11 b2 - m12 b1) / det, x1 = (M22 b1 - m12 b2) / det with det = m11 M22 - m12^2
       // (>= 0.19 for every theta2; condition number < 50), ONE float64 division per sub-step instead of three.  The
       // result differs from LAPACK's by a few float64 ulps (as the LU form did: dgesv scales by the reciprocal pivot), far
@@ -216,7 +209,6 @@ template <> struct Env<kTwoLink> {
       const double rdet = 1.0 / (m11 * M22 - m12 * m12);
       const double x2 = (m11 * b2 - m12 * b1) * rdet;
       const double x1 = (M22 * b1 - m12 * b2) * rdet;
-#endif
       o[0] = (float)((double)th1 + q1 * kDtD);
       o[1] = (float)((double)th2 + q2 * kDtD);
       o[2] = (float)((double)d1 + x1 * kDtD);
@@ -401,9 +393,7 @@ __device__ __forceinline__ void quad_polar_f32(float (&R)[9], float theta2) {
     const float c10 = cof(R[2], R[7], R[1], R[8]), c11 = cof(R[0], R[8], R[2], R[6]), c12 = cof(R[1], R[6], R[0], R[7]);
     const float c20 = cof(R[1], R[5], R[2], R[4]), c21 = cof(R[2], R[3], R[0], R[5]), c22 = cof(R[0], R[4], R[1], R[3]);
     const float det = __fmaf_rn(R[2], c02, __fmaf_rn(R[1], c01, R[0] * c00));
-#ifndef MSACL_QUAD_NO_REFLECT
     if (first && det < 0.0f) return false;
-#endif
     const float hid = 0.5f / det;                 // (an approximate reciprocal here measured 1.5 % slower end to end)
     R[0] = __fmaf_rn(c00, hid, 0.5f * R[0]); R[1] = __fmaf_rn(c01, hid, 0.5f * R[1]); R[2] = __fmaf_rn(c02, hid, 0.5f * R[2]);
     R[3] = __fmaf_rn(c10, hid, 0.5f * R[3]); R[4] = __fmaf_rn(c11, hid, 0.5f * R[4]); R[5] = __fmaf_rn(c12, hid, 0.5f * R[5]);

@@ -32,9 +32,6 @@ constexpr int GA_LBO = GM * 16, G_SBO = 128;
 //   converted B (weight gradient, un-packed weights):                warps 0-3 epilogue, warps 4-15 loaders (threads
 //       0..127 of the group own the A tile, 128..383 the B tile).
 constexpr int G_LOADERS = 384;
-#ifndef MSACL_GEMM_LOOKAHEAD
-#define MSACL_GEMM_LOOKAHEAD 3
-#endif
 constexpr int G_MMA_WARP = 16;
 constexpr int G_THREADS = 32 * (G_MMA_WARP + 1);
 
@@ -298,7 +295,7 @@ __global__ void __launch_bounds__(G_THREADS, 1) gemm_tc_kernel(msacl_gemm_t g) {
       //      stored (ncu, one-stage version: loader samples 46 % long-scoreboard, a stage cost ~4 k cycles against 1.5 k of
       //      UMMAs).  The buffers rotate by unrolling, never by register moves (a move of an in-flight load's destination
       //      would wait for it).
-      constexpr int G_LOOK = MSACL_GEMM_LOOKAHEAD;
+      constexpr int G_LOOK = 3;
       // fetch cursor: the position (tile, k stage) G_LOOK stages ahead of the one being stored
       int64_t ctile = blockIdx.x;
       GemmTile ctl;

@@ -23,8 +23,8 @@
 //   TMA warp          pre-split W2 k-step images (16 KB) global/L2 -> shared ring (cp.async.bulk).
 // All hand-offs are mbarriers (per-stage full/free for A and B, per-buffer full/free for H2, H1 full/free, X full,
 // logits); tcgen05.commit signals the ones the tensor pipe produces.
-#include <cstdlib>
-#include <type_traits>
+// The alternatives measured against this layout (two tiles per env warpgroup, a dedicated epilogue-1 group, 2 or 4 tile
+// slots) are in DESIGN.md §4.1.
 #include "common.cuh"
 #include "tcgen05.cuh"
 
@@ -66,34 +66,7 @@ __device__ __forceinline__ void wd_wait(void* bar, uint32_t parity, int site, ui
 #define TC_WAIT(bar, par, site, aux) tc::mbar_wait(bar, par)
 #endif
 
-#ifndef MSACL_TC_NS
-#define MSACL_TC_NS(ID) 3
-#endif
-// Tiles per env warpgroup (TPW).  1: a warpgroup owns one tile and keeps its env state in registers for all K steps.
-// 2: a warpgroup alternates between two tiles -- while the MLP of one runs it integrates the other -- with the env
-// state parked in its global arrays between steps (L2-resident: the tiles in flight of all CTAs are ~30 MB) and the
-// logits handed over through a per-CTA global scratch area (no shared memory left for 2 NS tiles).  The quadrotor is
-// bound by slots x (env-phase latency + MLP latency), not by any pipe; doubling the tiles in flight without doubling
-// the env threads' registers is what TPW = 2 buys.
-// Measured (round 2, QuadTracking, 2^21 envs x 16 steps): TPW = 2 is NOT faster (16.2 ms vs 15.4 ms per launch).  With the
-// warpgroups free-running, three copies of the ~50 KB env phase stream through the 32 KB instruction cache at once (ncu:
-// icc hit rate 78 %, gcc instruction requests 93 % of peak, 33 % of the env-phase samples `no_instruction`); with the
-// batch wait below the fetches are shared (icc 96 %, gcc 50 %) but the twelve env warps then contend for issue slots and
-// the FP64 pipe (math-pipe throttle 1.8 warps per issue): every arrangement tried -- (NS, TPW) = (3,1) (3,2) (2,2) (2,3)
-// (4,1) -- lands within 8 % of 14 k cycles per tile-step: the SM's instruction throughput for this mix of dependent
-// FP32 / FP64 / MUFU code at 5-6 resident warps per sub-partition (~0.5 IPC; profiles/r2_rollout_tc_tile_slot_experiments.md).
-// Kept as a build option (MSACL_TC_TPW=2); default 1.
-#ifndef MSACL_TC_TPW
-#define MSACL_TC_TPW(ID) 1
-#endif
-// Warps of a DEDICATED epilogue-1 group (E1).  0: the 8 epilogue warps run both epilogues of every tile-step one after the
-// other (epilogue 1 of t+1, then epilogue 2 of t).  8 / 4: epilogue 1 gets its own 8 warps (column halves, as before) / 4 warps
-// (whole rows), and the 8 warps behind them run epilogue 2 only -- the two epilogues of different tile-steps then overlap
-// instead of queueing in the same warps (role timers: the shared warps are busy 3.9 k + 6.4 k of the 14.4 k cycles per
-// tile-step and every hand-off in the MMA -> epilogue 1 -> MMA -> epilogue 2 chain waits for them).
-#ifndef MSACL_TC_E1
-#define MSACL_TC_E1(ID) 0
-#endif
+constexpr int TC_NS = 3;            // tile slots in flight per CTA = env warpgroups
 constexpr int TCM = 128;            // envs per tile
 constexpr int TC_HID = 256;
 constexpr int KC2 = 32;             // K per A stage
@@ -106,36 +79,22 @@ constexpr int B_HALF = TC_HID * KCB * 2;    // 8 KB  (b1 or b2 image of a stage)
 constexpr int A_LBO = TCM * 16, B_LBO = TC_HID * 16, SBO = 128;
 constexpr int X_HALF = TCM * 16 * 2;        // 4 KB  (x1 or x2: 128 rows x 16 k)
 constexpr int W1_HALF = TC_HID * 16 * 2;    // 8 KB
-// Launch geometry per number of tile slots in flight: NS env warpgroups + epilogue 1 + epilogue 2 +
-// {MMA, TMA, 2 idle warps}.  Registers are rebalanced with setmaxnreg (65536 per SM in total).  Per warp:
-// launch regs * warps >= sum of the budgets below, or setmaxnreg.inc never returns; and all four warps of a
-// warpgroup must execute the same setmaxnreg (the {MMA, TMA, idle, idle} group shares MISC_REGS).
-template <int NS, int E1 = 0> struct TcCfg;
-template <> struct TcCfg<3, 8> { static constexpr int THREADS = 1024, ENV_REGS = 80, EPI_REGS = 56, MISC_REGS = 32, NB = 3; };  // launch 64*32 = 2048 >= 12*80 + 16*56 + 4*32
-template <> struct TcCfg<3, 4> { static constexpr int THREADS = 896, ENV_REGS = 96, EPI_REGS = 56, MISC_REGS = 32, NB = 3; };   // launch 72*28 = 2016 >= 12*96 + 12*56 + 4*32
-template <> struct TcCfg<2> { static constexpr int THREADS = 640, ENV_REGS = 152, EPI_REGS = 64, MISC_REGS = 40, NB = 3; };   // launch 96*20 = 1920 >= 8*152 + 8*64 + 4*40
-template <> struct TcCfg<3> { static constexpr int THREADS = 768, ENV_REGS = 112, EPI_REGS = 56, MISC_REGS = 32, NB = 3; };   // launch 80*24 = 1920 = 12*112 + 8*56 + 4*32
-template <> struct TcCfg<4> { static constexpr int THREADS = 896, ENV_REGS = 88, EPI_REGS = 56, MISC_REGS = 40, NB = 2; };    // launch 72*28 = 2016 = 16*88 + 8*56 + 4*40; the 4th slot's 8 KB come out of the W2 ring
+// Launch geometry: TC_NS env warpgroups + 8 epilogue warps + {MMA, TMA, 2 idle warps}.  Registers are rebalanced with
+// setmaxnreg (65536 per SM in total).  Per warp: launch regs * warps >= sum of the budgets below, or setmaxnreg.inc never
+// returns; and all four warps of a warpgroup must execute the same setmaxnreg (the {MMA, TMA, idle, idle} group shares
+// TC_MISC_REGS).  Launch 80*24 = 1920 = 12*112 + 8*56 + 4*32.
+constexpr int TC_THREADS = 768, TC_ENV_REGS = 112, TC_EPI_REGS = 56, TC_MISC_REGS = 32;
 constexpr int W2P_BYTES = NCHB * 2 * B_HALF;   // 256 KB packed W2 (hi/lo k-step images)
 constexpr int W1P_BYTES = 2 * W1_HALF;
-// per-CTA global scratch behind the packed W2 image (TPW > 1): partial logits [tile slot][column half][8][128]
-constexpr int SCR_TILES = 8;
-constexpr int SCR_PER_TILE = 2 * 8 * TCM;
-constexpr int SCR_PER_CTA = SCR_TILES * SCR_PER_TILE;                  // 16384 floats = 64 KB
-constexpr bool tc_any_parked() {
-  return MSACL_TC_TPW(kVanderPol) > 1 || MSACL_TC_TPW(kPendulum) > 1 || MSACL_TC_TPW(kDuctedFan) > 1 || MSACL_TC_TPW(kTwoLink) > 1 ||
-         MSACL_TC_TPW(kSingleTrackCar) > 1 || MSACL_TC_TPW(kQuadTracking) > 1;
-}
-constexpr int64_t TC_SCRATCH_BYTES = tc_any_parked() ? (int64_t)kNumSMs * SCR_PER_CTA * 4 : 0;   // default build: none
 
 struct TcBars {
-  unsigned long long xfull[4], xfree[4], logits[8];
+  unsigned long long xfull[TC_NS], logits[TC_NS];
   unsigned long long h1full[2], h1free[2], h2full[2], h2free[2];   // per TMEM buffer
   unsigned long long afull[NCH], afree[NCH], bfull[NB_MAX], bfree[NB_MAX];
   uint32_t tmem_slot;
 };
 
-// The share of the tile list one CTA walks (TPW == 1; see the comment in the kernel): `share` contiguous tiles from `first`, in
+// The share of the tile list one CTA walks (see the comment in the kernel): `share` contiguous tiles from `first`, in
 // `rounds` rounds of per (+ 1 for the first `ex`) tiles.  Host + device: msacl_tc_tile_share() exposes the same arithmetic to the
 // CPU tests (every tile exactly once, round sizes <= NS and non-increasing).
 struct TcShare {
@@ -157,19 +116,19 @@ struct TcShare {
 // operand descriptors' K-block stride (LBO) points at one shared zero block instead.  That and the narrower W3 (2A <= 4)
 // free the shared memory for a fourth W2 ring stage.
 template <int ID> __host__ __device__ constexpr bool tc_two_kblocks() { return Env<ID>::D + 1 > 8; }
-template <int ID, int NS> __host__ __device__ constexpr int tc_ring_depth() { return NS == 4 ? 2 : (tc_two_kblocks<ID>() ? 3 : 4); }
+template <int ID> __host__ __device__ constexpr int tc_ring_depth() { return tc_two_kblocks<ID>() ? 3 : 4; }
 template <int ID> __host__ __device__ constexpr int tc_w3_stride() { return 2 * Env<ID>::A > 4 ? 8 : 4; }
 
-template <int ID, int NS>
+template <int ID>
 struct TcSmem {
   static constexpr bool X2 = tc_two_kblocks<ID>();
-  static constexpr int NB = tc_ring_depth<ID, NS>();
+  static constexpr int NB = tc_ring_depth<ID>();
   static constexpr int XH = X2 ? X_HALF : X_HALF / 2;          // bytes of the hi (or lo) image of a slot's X operand
   static constexpr int W1H = X2 ? W1_HALF : W1_HALF / 2;       // bytes of the hi (or lo) image of the W1|b1 operand
   alignas(128) unsigned char bstage[NB][2 * B_HALF];     //  48 KB (box envs: 64 KB)
   alignas(128) unsigned char astage[NCH][2 * A_HALF];    // 128 KB
   alignas(128) unsigned char w1p[2 * W1H];               //  16 KB (box envs: 8 KB)
-  alignas(128) unsigned char xop[NS][2 * XH];            //   8 KB (4 KB) per env warpgroup; TPW == 1: doubles as the slot's logits
+  alignas(128) unsigned char xop[TC_NS][2 * XH];         //   8 KB (4 KB) per env warpgroup; doubles as the slot's logits
   alignas(128) unsigned char zeros[X2 ? 128 : W1_HALF / 2];   // shared all-zero second K block (box envs)
   alignas(16) float w3t[TC_HID * tc_w3_stride<ID>()];   // layer-3 weights transposed: [unit n][output j] (zero padded)
   alignas(16) float b2[TC_HID];
@@ -236,34 +195,26 @@ __global__ void tc_pack_actor_kernel(msacl_actor_t actor, int D, unsigned char* 
   }
 }
 
-template <int ID, int NS, int TPW, int E1>
-__global__ void __launch_bounds__(TcCfg<NS, E1>::THREADS, 1)
+template <int ID>
+__global__ void __launch_bounds__(TC_THREADS, 1)
 rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char* __restrict__ w1p_g,
-                  const unsigned char* __restrict__ w2p_g, float* __restrict__ scratch, int K, uint32_t step_base, int n_step,
+                  const unsigned char* __restrict__ w2p_g, int K, uint32_t step_base, int n_step,
                   float reward_scale, float cost_scale, const float* __restrict__ eps, int deterministic, msacl_transitions_t out,
                   double* stats) {
   using E = Env<ID>;
-  using S = TcSmem<ID, NS>;
-  using CFG = TcCfg<NS, E1>;
-  static_assert(E1 == 0 || ((E1 == 4 || E1 == 8) && TPW == 1), "dedicated epilogue-1 group: 4 or 8 warps, one tile per env warpgroup");
+  using S = TcSmem<ID>;
   constexpr int D = E::D, A = E::A, A2 = 2 * A;
-  constexpr int NT = NS * TPW;                 // tiles in flight per CTA ("group"); tile slot s belongs to warpgroup s % NS
-  constexpr bool PARK = TPW > 1;
-  // env state parked in global memory between steps, logits through global scratch
-  static_assert(NT <= SCR_TILES && A2 <= 8, "scratch layout");
-  constexpr int TC_THREADS = CFG::THREADS, NB = S::NB, XH = S::XH, W1H = S::W1H, W3S = tc_w3_stride<ID>();
+  constexpr int NS = TC_NS;                    // tiles in flight per CTA ("group"); tile slot s belongs to warpgroup s % NS
+  constexpr int NB = S::NB, XH = S::XH, W1H = S::W1H, W3S = tc_w3_stride<ID>();
   constexpr bool X2 = S::X2;
-  constexpr int W_EPI1 = 4 * NS, W_EPI2 = W_EPI1 + E1, W_MMA = W_EPI2 + 8, W_TMA = W_MMA + 1;
-  constexpr int NC1 = E1 == 4 ? NCH : NCH / 2;      // A stages a warp of epilogue 1 fills per tile-step
+  constexpr int W_EPI1 = 4 * NS, W_MMA = W_EPI1 + 8, W_TMA = W_MMA + 1;
   static_assert(D < 16, "layer-1 K block holds obs + bias column");
-  static_assert(A2 * TCM * 4 <= XH && ((A2 + 1) / 2) * 2 * TCM * 4 <= XH, "logits and partial sums alias the two halves of the X-operand region (TPW == 1)");
+  static_assert(A2 * TCM * 4 <= XH && ((A2 + 1) / 2) * 2 * TCM * 4 <= XH, "logits and partial sums alias the two halves of the X-operand region");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   S& sm = *reinterpret_cast<S*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  // TPW == 1: a slot's logits live in its X-operand region (free between layer 1 and the next write_xop);
-  // TPW > 1: in this CTA's global scratch (the X region is shared by the warpgroup's tiles)
-  float* const scr = PARK ? scratch + (size_t)blockIdx.x * SCR_PER_CTA : nullptr;
-  auto logits_of = [&](int s) { return PARK ? scr + s * SCR_PER_TILE : reinterpret_cast<float*>(sm.xop[s]); };   // [2A][128] f32
+  // a slot's logits live in its X-operand region (free between layer 1 and the next write_xop)
+  auto logits_of = [&](int s) { return reinterpret_cast<float*>(sm.xop[s]); };   // [2A][128] f32
 
   // ---- one-time setup
   // W1|b1 images: the packed global buffer always holds both K blocks per image; box envs keep only the first
@@ -277,10 +228,10 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
   if (tid < 8) sm.b3[tid] = tid < A2 ? actor.b3[tid] : 0.f;
   if (tid == 0) {
     TcBars& b = sm.bars;
-    for (int s = 0; s < NS; ++s) { tc::mbar_init(&b.xfull[s], TCM); tc::mbar_init(&b.xfree[s], 1); }
-    for (int s = 0; s < NT; ++s) tc::mbar_init(&b.logits[s], PARK ? 2 * TCM : TCM);   // PARK: both column halves deliver
+    for (int s = 0; s < NS; ++s) tc::mbar_init(&b.xfull[s], TCM);
+    for (int s = 0; s < NS; ++s) tc::mbar_init(&b.logits[s], TCM);
     for (int i = 0; i < 2; ++i) {
-      tc::mbar_init(&b.h1full[i], 1); tc::mbar_init(&b.h1free[i], E1 == 4 ? TCM : 2 * TCM);     // drained by all warps of epilogue 1
+      tc::mbar_init(&b.h1full[i], 1); tc::mbar_init(&b.h1free[i], 2 * TCM);     // drained by all warps of epilogue 1
       tc::mbar_init(&b.h2full[i], 1); tc::mbar_init(&b.h2free[i], 2 * TCM);
     }
     for (int i = 0; i < NCH; ++i) { tc::mbar_init(&b.afull[i], TCM); tc::mbar_init(&b.afree[i], 1); }
@@ -295,44 +246,35 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
   const uint32_t tmem = sm.bars.tmem_slot;     // buffer b of tile-step t (b = t & 1) = columns [256 b, 256 b + 256)
 
   const int64_t num_tiles = (st.n + TCM - 1) / TCM;
-  // Groups ("pairs") of up to NT tiles in flight.  A CTA walks the group ids cta, cta + G, cta + 2 G, ... (G = gridDim.x).
-  // TPW == 1: the tiles are dealt to the CTAs in contiguous BALANCED shares -- CTA b owns T / G (+ 1) tiles and walks them in
-  // ceil(share / NT) rounds of share / rounds (+ 1) tiles, the larger rounds first (so a warpgroup that has no tile in a round
+  // Groups ("pairs") of up to NS tiles in flight.  A CTA walks the group ids cta, cta + G, cta + 2 G, ... (G = gridDim.x).
+  // The tiles are dealt to the CTAs in contiguous BALANCED shares -- CTA b owns T / G (+ 1) tiles and walks them in
+  // ceil(share / NS) rounds of share / rounds (+ 1) tiles, the larger rounds first (so a warpgroup that has no tile in a round
   // has none in the later ones, and every earlier round of an active warpgroup was a full K steps: x_index below).  Cutting the
-  // tile list into fixed groups of NT instead leaves most SMs idle for half the launch when the tile count is a small
+  // tile list into fixed groups of NS instead leaves most SMs idle for half the launch when the tile count is a small
   // multiple of the SM count: 65 536 envs = 512 tiles = 171 groups of 3 on 148 SMs are TWO rounds of 3 tiles for 23 CTAs and one
   // for the rest; balanced, 68 CTAs run two rounds of 2 tiles and 80 one round of 3.  Results do not depend on the mapping
-  // (the RNG streams are keyed by the global env id).  TPW > 1 keeps fixed groups of NT tiles.
+  // (the RNG streams are keyed by the global env id).
   const int64_t G = gridDim.x, cta = blockIdx.x;
-  const TcShare sh(num_tiles, G, cta, NT);
-  const int64_t num_pairs = PARK ? (num_tiles + NT - 1) / NT : cta + (int64_t)sh.rounds * G;      // bound of `for (pair = cta; pair < num_pairs; pair += G)`
-  auto tiles_in_pair = [&](int64_t pair) -> int {
-    if (PARK) return (int)((num_tiles - NT * pair) < NT ? (num_tiles - NT * pair) : NT);
-    return sh.tiles_in_round((int)(pair - cta) / (int)G);      // (32-bit division: round index = tiles / G at most)
-  };
-  auto first_tile = [&](int64_t pair) -> int64_t {
-    if (PARK) return NT * pair;
-    return sh.first_tile_of_round((int)(pair - cta) / (int)G);
-  };
+  const TcShare sh(num_tiles, G, cta, NS);
+  const int64_t num_pairs = cta + (int64_t)sh.rounds * G;      // bound of `for (pair = cta; pair < num_pairs; pair += G)`
+  // (32-bit division: round index = tiles / G at most)
+  auto tiles_in_pair = [&](int64_t pair) -> int { return sh.tiles_in_round((int)(pair - cta) / (int)G); };
+  auto first_tile = [&](int64_t pair) -> int64_t { return sh.first_tile_of_round((int)(pair - cta) / (int)G); };
   // X operands are written per warpgroup: group pi (all but the last are full), step k, tile slot s -> running index
   auto tiles_of_wg = [&](int w, int nt) { return nt > w ? (nt - w - 1) / NS + 1 : 0; };
-  auto x_index = [&](uint32_t pi, int k, int s, int nt) { return pi * (uint32_t)(TPW * K) + (uint32_t)(k * tiles_of_wg(s % NS, nt) + s / NS); };
+  auto x_index = [&](uint32_t pi, int k, int s, int nt) { return pi * (uint32_t)K + (uint32_t)(k * tiles_of_wg(s % NS, nt) + s / NS); };
 
   if (warp < W_EPI1) {
     // =========================== env warps ===========================
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(CFG::ENV_REGS));
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(TC_ENV_REGS));
     const int w = warp >> 2;                 // env warpgroup: tile slots w, w + NS, ...
     const int r = tid & (TCM - 1);
-    uint32_t xcount = 0;                     // X operands this warpgroup has written
     uint32_t lcount = 0;                     // logits deliveries each of its tile slots has consumed
     float st_ep = 0.f, st_ret = 0.f, st_len = 0.f, st_term = 0.f, st_trunc = 0.f;
     auto write_xop = [&](const float* obs, bool valid) {
       float v[16];
 #pragma unroll
       for (int k = 0; k < 16; ++k) v[k] = (k < D) ? (valid ? obs[k < D ? k : 0] : 0.f) : (k == D ? 1.f : 0.f);
-      // (TPW > 1) the region is shared by the warpgroup's tiles: layer 1 of the previous X operand must have read it
-      if (PARK && xcount > 0) TC_WAIT(&sm.bars.xfree[w], (xcount - 1) & 1, 14, xcount);
-      ++xcount;
 #pragma unroll
       for (int kb = 0; kb < (X2 ? 2 : 1); ++kb) {
         float wv[8];
@@ -364,7 +306,6 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         for (int s = w; s < nt; s += NS) {
         const int64_t gi = (tile0 + s) * TCM + r;
         const bool owner = gi < st.n;
-        if (PARK && owner) e.load(st, gi);     // issued in front of the logits wait: the L2 round trip hides behind it
         // the action noise of this step does not depend on the logits: draw it while the tile's MLP is still running
         float z[4] = {0.f, 0.f, 0.f, 0.f};
         if (owner && !deterministic) {
@@ -378,31 +319,14 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
 #ifdef MSACL_TC_TIMING
         const long long t_w0 = clock64();
 #endif
-        if constexpr (PARK) {
-          // wait for the logits of ALL tiles of this batch (slots sub*NS .. sub*NS + NS - 1), so that the env warpgroups run
-          // the (long, straight-line) env phase in step and share its instruction-cache lines: one warpgroup per tile
-          // streaming ~50 KB of code on its own saturates the GPC-level instruction cache (ncu: gcc instruction
-          // requests 81-93 % of peak, icc hit rate = the 75 % that the four warps of one warpgroup share)
-          const int s0 = s - w;
-#pragma unroll
-          for (int j = 0; j < NS; ++j)
-            if (s0 + j < nt) TC_WAIT(&sm.bars.logits[s0 + j], lcount & 1, 1, lcount);
-        } else {
-          TC_WAIT(&sm.bars.logits[s], lcount & 1, 1, lcount);
-        }
+        TC_WAIT(&sm.bars.logits[s], lcount & 1, 1, lcount);
+        // the logits of this slot were written into its X-operand region (free between layer 1 and the next
+        // write_xop): take them into registers, then a slot-wide barrier so that no thread of the slot can overwrite
+        // them with its next observation before every thread has read its own
         float lg[A2];
-        if constexpr (PARK) {
-          // written with st.global.cg by the epilogue warps of this CTA before their (release) arrive on the barrier
 #pragma unroll
-          for (int j = 0; j < A2; ++j) lg[j] = __ldcg(logits_of(s) + j * TCM + r) + __ldcg(logits_of(s) + SCR_PER_TILE / 2 + j * TCM + r);
-        } else {
-          // the logits of this slot were written into its X-operand region (free between layer 1 and the next
-          // write_xop): take them into registers, then a slot-wide barrier so that no thread of the slot can overwrite
-          // them with its next observation before every thread has read its own
-#pragma unroll
-          for (int j = 0; j < A2; ++j) lg[j] = logits_of(s)[j * TCM + r];
-          asm volatile("bar.sync %0, 128;" ::"r"(1 + w) : "memory");
-        }
+        for (int j = 0; j < A2; ++j) lg[j] = logits_of(s)[j * TCM + r];
+        asm volatile("bar.sync %0, 128;" ::"r"(1 + w) : "memory");
 #ifdef MSACL_TC_TIMING
         const long long t_w1 = clock64();
 #endif
@@ -473,7 +397,6 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
           if (out.done) out.done[row] = done ? 1 : 0;
           if (out.logp) out.logp[row] = logp;
           if (out.emit) out.emit[row] = emit ? 1 : 0;
-          if (PARK) e.store(st, gi);
         } else if (k + 1 < K) {
           write_xop(e.obs(), false);
         }
@@ -488,10 +411,8 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         }
         ++lcount;
       }
-      if constexpr (!PARK) {
-        const int64_t gi = (tile0 + w) * TCM + r;
-        if (gi < st.n) e.store(st, gi);
-      }
+      const int64_t gi = (tile0 + w) * TCM + r;
+      if (gi < st.n) e.store(st, gi);
     }
     if (stats) {
       float v[5] = {st_ep, st_ret, st_len, st_term, st_trunc};
@@ -512,14 +433,12 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
     // Job order per tile-step t (groups of >= 2 slots): epilogue 1 of t+1 (it trails layer 2 of t stage by stage), then
     // epilogue 2 of t (while layer 2 of t+1 runs).  With a single slot the X operand of t+1 needs the logits of t, so
     // the order is swapped.
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(CFG::EPI_REGS));
-    // E1 > 0: warps [W_EPI1, W_EPI2) run epilogue 1 only, [W_EPI2, W_MMA) epilogue 2 only
-    const bool first_group = E1 == 0 || warp < W_EPI2;
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(TC_EPI_REGS));
     const int q = warp & 3;
-    const int h = first_group ? (E1 == 4 ? 0 : (warp - W_EPI1) >> 2) : (warp - W_EPI2) >> 2;      // column half
+    const int h = (warp - W_EPI1) >> 2;      // column half
     const int r = q * 32 + lane;
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-    const bool timer = lane == 0 && (warp == W_EPI1 || (E1 > 0 && warp == W_EPI2));
+    const bool timer = lane == 0 && warp == W_EPI1;
     auto epi1 = [&](uint32_t t1) {
       const uint32_t buf = t1 & 1u, tmem_b = tmem + buf * 256u;
       TC_T0(t_a);
@@ -528,7 +447,7 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
       if (timer) TC_ACC(8, t_a);                      // epi1: wait for H1
       TC_T0(t_b);
 #pragma unroll 1
-      for (int cc = 0; cc < NC1; ++cc) {
+      for (int cc = 0; cc < NCH / 2; ++cc) {
         const int c = h * (NCH / 2) + cc;
         TC_T0(t_c);
         if (t1 > 0) TC_WAIT(&sm.bars.afree[c], (t1 - 1) & 1, 3, t1);   // layer 2 of the previous tile-step is done with stage c
@@ -536,7 +455,7 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         uint32_t v[32];
         tc::tmem_ld32(tmem_b + lane_addr + (uint32_t)(c * 32), v);
         tc::tmem_ld_wait();
-        if (cc == NC1 - 1) { tc::tc_fence_before(); tc::mbar_arrive(&sm.bars.h1free[buf]); }   // layer 2 may overwrite the buffer
+        if (cc == NCH / 2 - 1) { tc::tc_fence_before(); tc::mbar_arrive(&sm.bars.h1free[buf]); }   // layer 2 may overwrite the buffer
         unsigned char* base = sm.astage[c] + r * 16;
 #pragma unroll
         for (int kb = 0; kb < 4; ++kb) {
@@ -594,67 +513,38 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         }
       }
       // combine the two column halves: rows of quadrant q are shared by warps (q, half 0) and (q, half 1)
-      // combine the two column halves: rows of quadrant q are shared by warps (q, half 0) and (q, half 1)
-      if constexpr (PARK) {
-        // both halves hand their partial logits to the slot's env warps through this CTA's global scratch (L2-only stores,
-        // ordered by the release-arrive below); the env thread adds them (half 0 + half 1, the order of the TPW == 1 path)
-        float* lgs = logits_of(s) + h * (SCR_PER_TILE / 2);
+      float* part = reinterpret_cast<float*>(sm.xop[s] + XH);      // second half of the slot's X-operand region
+      float* lgs = logits_of(s);
+      if (h == 1) {
 #pragma unroll
         for (int p = 0; p < NP; ++p) {
           float lo, hi;
           unpack2(acc[p], lo, hi);
-          __stcg(&lgs[(2 * p) * TCM + r], lo);
-          if (2 * p + 1 < A2) __stcg(&lgs[(2 * p + 1) * TCM + r], hi);
+          part[(2 * p) * TCM + r] = lo;
+          part[(2 * p + 1) * TCM + r] = hi;
+        }
+      }
+      asm volatile("bar.sync %0, 64;" ::"r"(4 + q) : "memory");
+      if (h == 0) {
+#pragma unroll
+        for (int p = 0; p < NP; ++p) {
+          float lo, hi;
+          unpack2(acc[p], lo, hi);
+          lgs[(2 * p) * TCM + r] = lo + part[(2 * p) * TCM + r];
+          if (2 * p + 1 < A2) lgs[(2 * p + 1) * TCM + r] = hi + part[(2 * p + 1) * TCM + r];
         }
         tc::mbar_arrive(&sm.bars.logits[s]);
-      } else {
-        float* part = reinterpret_cast<float*>(sm.xop[s] + XH);      // second half of the slot's X-operand region
-        float* lgs = logits_of(s);
-        if (h == 1) {
-#pragma unroll
-          for (int p = 0; p < NP; ++p) {
-            float lo, hi;
-            unpack2(acc[p], lo, hi);
-            part[(2 * p) * TCM + r] = lo;
-            part[(2 * p + 1) * TCM + r] = hi;
-          }
-        }
-        asm volatile("bar.sync %0, 64;" ::"r"(4 + q) : "memory");
-        if (h == 0) {
-#pragma unroll
-          for (int p = 0; p < NP; ++p) {
-            float lo, hi;
-            unpack2(acc[p], lo, hi);
-            lgs[(2 * p) * TCM + r] = lo + part[(2 * p) * TCM + r];
-            if (2 * p + 1 < A2) lgs[(2 * p + 1) * TCM + r] = hi + part[(2 * p + 1) * TCM + r];
-          }
-          tc::mbar_arrive(&sm.bars.logits[s]);
-        }
       }
       if (timer) TC_ACC(12, t_b);                     // epi2: compute
     };
     uint32_t ts = 0;
-    if constexpr (E1 > 0) {
-      // two independent groups: each walks the tile-steps in order; the hand-offs with the MMA thread are the only coupling
-      for (int64_t pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
-        const int nt = tiles_in_pair(pair);
-        for (int k = 0; k < K; ++k)
-          for (int s = 0; s < nt; ++s, ++ts) {
-            if (first_group) epi1(ts);
-            else epi2(ts, s);
-          }
-      }
-    } else
     for (int64_t pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
       const int nt = tiles_in_pair(pair);
       for (int k = 0; k < K; ++k)
         for (int s = 0; s < nt; ++s, ++ts) {
           if (ts == 0) epi1(0u);
           const bool has_next = !(s + 1 == nt && k + 1 == K && pair + (int64_t)gridDim.x >= num_pairs);
-          // PARK: the env warpgroups wait for the logits of a whole batch of NS tiles, so the X operand of the successor
-          // depends on THIS tile-step's logits when the group has a single batch, and at the last tile-step of a group
-          // (the first X operand of the next group is written after the warpgroup's last env step)
-          const bool epi2_first = PARK ? (nt <= NS || (s + 1 == nt && k + 1 == K)) : (nt <= 1);
+          const bool epi2_first = nt <= 1;
           if (!epi2_first) {
             if (has_next) epi1(ts + 1);
             epi2(ts, s);
@@ -666,7 +556,7 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
     }
   } else {
     // (setmaxnreg must be executed with the same value by all four warps of a warpgroup)
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(CFG::MISC_REGS));
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(TC_MISC_REGS));
     if (warp == W_MMA) {
     // =========================== MMA issuer ===========================
     if (tc::elect_one()) {
@@ -701,7 +591,6 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         tc::umma_bf16(tmem_b, dx1, dw2, idesc, 1u);
         tc::umma_bf16(tmem_b, dx2, dw1, idesc, 1u);
         tc::umma_commit(&sm.bars.h1full[t1 & 1]);
-        if (PARK) tc::umma_commit(&sm.bars.xfree[s % NS]);     // the warpgroup may write its next X operand
       };
       uint32_t ts = 0, pi = 0;                        // tile-step counter, local group counter
       for (int64_t pair = blockIdx.x; pair < num_pairs; pair += gridDim.x, ++pi) {
@@ -800,14 +689,14 @@ extern "C" int msacl_rollout_tc_set_max_ctas(int32_t max_ctas) {
 
 extern "C" int msacl_tc_tile_share(int64_t n_envs, int32_t grid, int32_t cta, int64_t* out) {
   if (n_envs <= 0 || grid <= 0 || cta < 0 || cta >= grid || !out) { set_error("tc_tile_share: bad argument"); return MSACL_ERR_BAD_ARG; }
-  const TcShare sh((n_envs + TCM - 1) / TCM, grid, cta, 3);
+  const TcShare sh((n_envs + TCM - 1) / TCM, grid, cta, TC_NS);
   out[0] = sh.first; out[1] = sh.share; out[2] = sh.rounds; out[3] = sh.per; out[4] = sh.ex;
   return MSACL_OK;
 }
 
 extern "C" int msacl_tc_pack_bytes(int64_t* w1p_bytes, int64_t* w2p_bytes) {
   if (w1p_bytes) *w1p_bytes = W1P_BYTES;
-  if (w2p_bytes) *w2p_bytes = W2P_BYTES + TC_SCRATCH_BYTES;     // packed W2 images + the rollout kernel's per-CTA scratch
+  if (w2p_bytes) *w2p_bytes = W2P_BYTES;
   return MSACL_OK;
 }
 
@@ -830,28 +719,15 @@ extern "C" int msacl_rollout_fused_tc(const msacl_env_state_t* st, const msacl_a
       set_error("rollout_fused_tc: transition obs/obs2/act rows must be aligned to their vector width (16 B if the row length is a multiple of 4 floats, 8 B if even)");
       return MSACL_ERR_BAD_ARG;
     }
-    constexpr int NS = MSACL_TC_NS(ID);      // env warpgroups
-    constexpr int TPW = MSACL_TC_TPW(ID);    // tiles per warpgroup: NS * TPW tiles in flight per CTA
-    constexpr int E1_DEFAULT = MSACL_TC_E1(ID);      // warps of a dedicated epilogue-1 group (0: shared epilogue warps; needs NS == 3)
-    static_assert(sizeof(TcSmem<ID, NS>) + 128 <= 232448, "shared-memory layout exceeds the 227 KB per-CTA limit");
-    const int64_t groups = TPW == 1 ? tiles : (tiles + NS * TPW - 1) / (NS * TPW);      // TPW == 1: balanced shares, every CTA owns >= 1 tile
+    static_assert(sizeof(TcSmem<ID>) + 128 <= 232448, "shared-memory layout exceeds the 227 KB per-CTA limit");
     const int64_t cap = g_tc_max_ctas > 0 ? g_tc_max_ctas : kNumSMs;
-    const unsigned grid = (unsigned)(groups < cap ? groups : cap);
-    const size_t smem = sizeof(TcSmem<ID, NS>) + 128;
-    // the scratch area behind the W2 images is written by the kernel (the ABI hands the buffer over as const because the
-    // images are; one launch at a time may use a given buffer)
-    float* scratch = reinterpret_cast<float*>(const_cast<unsigned char*>((const unsigned char*)w2p) + W2P_BYTES);
-    auto launch = [&](auto e1_tag) -> int {
-      constexpr int E1 = decltype(e1_tag)::value;
-      auto kern = rollout_tc_kernel<ID, NS, TPW, E1>;
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e != cudaSuccess) { set_error("rollout_fused_tc: smem attr (%zu B): %s", smem, cudaGetErrorString(e)); return MSACL_ERR_CUDA; }
-      kern<<<grid, TcCfg<NS, E1>::THREADS, smem, (cudaStream_t)stream>>>(*st, *actor, (const unsigned char*)w1p, (const unsigned char*)w2p, scratch, K,
-                                                                         step_base, n_step, reward_scale, cost_scale, eps, deterministic, *out, stats);
-      return MSACL_OK;
-    };
-    const int rc = launch(std::integral_constant<int, E1_DEFAULT>{});
-    if (rc != MSACL_OK) return rc;
+    const unsigned grid = (unsigned)(tiles < cap ? tiles : cap);      // balanced shares: every CTA owns >= 1 tile
+    const size_t smem = sizeof(TcSmem<ID>) + 128;
+    auto kern = rollout_tc_kernel<ID>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) { set_error("rollout_fused_tc: smem attr (%zu B): %s", smem, cudaGetErrorString(e)); return MSACL_ERR_CUDA; }
+    kern<<<grid, TC_THREADS, smem, (cudaStream_t)stream>>>(*st, *actor, (const unsigned char*)w1p, (const unsigned char*)w2p, K,
+                                                           step_base, n_step, reward_scale, cost_scale, eps, deterministic, *out, stats);
   });
   return check_launch("rollout_fused_tc");
 }

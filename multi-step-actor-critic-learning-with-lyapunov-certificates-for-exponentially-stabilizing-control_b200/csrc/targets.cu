@@ -123,9 +123,6 @@ lyapunov_risk_kernel(int64_t B, int n, int D_rt, const float* __restrict__ obs, 
   }
 }
 
-#ifndef MSACL_LYA_MINB
-#define MSACL_LYA_MINB 2
-#endif
 // All-lanes-live variant: a warp walks tiles of 32 P consecutive (window, step) elements, P = n / gcd(n, 32), so that a tile
 // holds whole windows (n = 20: 160 elements = 8 windows in 5 passes; n = 16: 2 windows in 1 pass).  Lane l of pass p owns
 // element 32 p + l of the tile -- coalesced loads, every lane busy (the warp-per-window kernel above keeps only n of 32
@@ -135,7 +132,7 @@ lyapunov_risk_kernel(int64_t B, int n, int D_rt, const float* __restrict__ obs, 
 // a segmented suffix sum plus the continuation at lane 0 of the next pass.  Same arithmetic per element as the kernel above; only the association of the cumprod / window sums
 // differs for windows that straddle two passes.
 template <int WPB, int P, int DT>
-__global__ void __launch_bounds__(WPB * 32, MSACL_LYA_MINB)
+__global__ void __launch_bounds__(WPB * 32, 2)
 lyapunov_risk_striped_kernel(int64_t B, int n, const float* __restrict__ obs, const float* __restrict__ obs2,
                              const float* __restrict__ logp_new, const float* __restrict__ logp_old,
                              const float* __restrict__ lya_obs, const float* __restrict__ lya_obs2,

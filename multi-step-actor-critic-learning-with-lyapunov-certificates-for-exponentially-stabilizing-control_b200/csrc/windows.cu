@@ -78,7 +78,7 @@ template <> struct ObsVec<2> { using type = float2; };
 template <> struct ObsVec<1> { using type = float; };
 
 // One warp copies one n-step window out of the [T][n][.] transition store into entry `slot` of a [.][n_step][.] window
-// array (the replay ring of window_scatter_kernel, or the sampled batch of window_gather_indexed_kernel).
+// array (the sampled batch of window_gather_indexed_kernel and window_sample_indexed_kernel).
 // A window's rows come from ns transition slices (stride n rows), its destination entry is contiguous per field.  Work
 // items are OW-float vectors of the obs / obs2 rows (OW = 4, 2 or 1: the widest that divides obs_dim), scalars of the act
 // rows, and one lane per row for the four per-step scalars.  The item -> (row, offset) map is the same for every
@@ -111,10 +111,7 @@ struct WindowCopier {
     float* dob = ring.obs + slot * ns * D;
     float* dob2 = ring.obs2 + slot * ns * D;
     float* da = ring.act + slot * ns * A;
-#ifndef MSACL_SCATTER_REGPATH
-#define MSACL_SCATTER_REGPATH 1
-#endif
-    if (MSACL_SCATTER_REGPATH && nv <= 32 * SC_IT && na <= 32 * SC_IT) {
+    if (nv <= 32 * SC_IT && na <= 32 * SC_IT) {
       // every load of the window is issued before the first store (one memory round trip per window)
       VecT vo[SC_IT], vo2[SC_IT];
       float va[SC_IT], vr = 0.f, vc = 0.f, vl = 0.f;
@@ -187,9 +184,6 @@ struct WindowCopier {
   }
 };
 
-#ifndef MSACL_SCATTER_GROUP
-#define MSACL_SCATTER_GROUP 8
-#endif
 // G windows per warp, 32 / G lanes each (window_scatter_kernel; described for G = 4).  The windows a block stores are consecutive in (t, env)
 // order, so the four windows of a warp are -- almost always -- four ADJACENT envs at the same step: for a given row the four
 // 8-lane groups then read one contiguous piece of the transition store (TwoLink: 4 x 16 B = two full sectors) instead of 20
@@ -315,21 +309,12 @@ window_scatter_kernel(msacl_transitions_t tr, int H, int64_t n, int64_t total_fl
   }
   __syncthreads();
   const int num = s_num;
-#ifdef MSACL_SCATTER_ONE_PER_WARP
-  WindowCopier<W> cp(tr, n, ring, lane);
-  for (int w = warp; w < num; w += WB / 32) {
-    const int64_t slot = s_slot[w];
-    if (slot < 0) continue;
-    cp.copy(s_src[w], slot);
-  }
-#else
-  constexpr int G = MSACL_SCATTER_GROUP;                 // windows per warp
+  constexpr int G = 8;                 // windows per warp
   WindowCopier4<W, G> cp(tr, n, ring, lane);
   for (int w0 = warp * G; w0 < num; w0 += (WB / 32) * G) {
     const int w = w0 + lane / (32 / G);
     cp.copy(w < num ? s_src[w] : 0, w < num ? s_slot[w] : -1);
   }
-#endif
 }
 
 // ---- index-based window store (SURVEY.md 8f-1): a window is the flat position of its newest transition in the

@@ -12,31 +12,21 @@ except Exception:
     pass
 D = int(os.environ.get("D", 4))
 NS = [int(x) for x in os.environ.get("N", "8,16,20,24,32").split(",")]
-# optional arguments: run-time variants "VAR=v[,VAR2=v2]" (environment variables the library reads at launch time; "-" = none)
-VARIANTS = sys.argv[1:] or ["-"]
-for variant in VARIANTS:
-  keys = []
-  if variant != "-":
-      for kv in variant.split(","):
-          k, v = kv.split("="); os.environ[k] = v; keys.append(k)
-      print("==", variant, flush=True)
-  for n in NS:
-      B = (1 << 20) * 20 // n
-      g = torch.Generator(device="cuda").manual_seed(0)
-      r = lambda *s: torch.randn(*s, device="cuda", generator=g)
-      obs, obs2, lpn, lpo, v1, v2 = r(B, n, D) * 0.5, r(B, n, D) * 0.5, r(B, n), r(B, n), r(B, n).abs(), r(B, n).abs()
-      coef = tg.Coefficients(n)
-      parts = torch.empty(3, dtype=torch.float64, device="cuda"); g1, g2 = torch.empty_like(v1), torch.empty_like(v2)
-      fn = lambda: _lib.check(lib.msacl_lyapunov_risk(B, n, D, obs.data_ptr(), obs2.data_ptr(), lpn.data_ptr(), lpo.data_ptr(), v1.data_ptr(),
-                                                      v2.data_ptr(), coef.son.data_ptr(), coef.diff.data_ptr(), coef.sl.data_ptr(), coef.alpha1,
-                                                      coef.alpha2, 10.0, 1.0, parts.data_ptr(), g1.data_ptr(), g2.data_ptr(), None, None, st))
-      for _ in range(3): fn()
-      a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-      torch.cuda.synchronize(); a.record()
-      for _ in range(20): fn()
-      b.record(); torch.cuda.synchronize()
-      ms = a.elapsed_time(b) / 20
-      gbs = B * n * 4 * (2 * D + 6) / ms / 1e6
-      print(f"n {n} D {D} ms {ms:.4f} GB/s {gbs:.0f} frac {gbs / HBM:.3f}", flush=True)
-  for k in keys:
-      del os.environ[k]
+for n in NS:
+    B = (1 << 20) * 20 // n
+    g = torch.Generator(device="cuda").manual_seed(0)
+    r = lambda *s: torch.randn(*s, device="cuda", generator=g)
+    obs, obs2, lpn, lpo, v1, v2 = r(B, n, D) * 0.5, r(B, n, D) * 0.5, r(B, n), r(B, n), r(B, n).abs(), r(B, n).abs()
+    coef = tg.Coefficients(n)
+    parts = torch.empty(3, dtype=torch.float64, device="cuda"); g1, g2 = torch.empty_like(v1), torch.empty_like(v2)
+    fn = lambda: _lib.check(lib.msacl_lyapunov_risk(B, n, D, obs.data_ptr(), obs2.data_ptr(), lpn.data_ptr(), lpo.data_ptr(), v1.data_ptr(),
+                                                    v2.data_ptr(), coef.son.data_ptr(), coef.diff.data_ptr(), coef.sl.data_ptr(), coef.alpha1,
+                                                    coef.alpha2, 10.0, 1.0, parts.data_ptr(), g1.data_ptr(), g2.data_ptr(), None, None, st))
+    for _ in range(3): fn()
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.synchronize(); a.record()
+    for _ in range(20): fn()
+    b.record(); torch.cuda.synchronize()
+    ms = a.elapsed_time(b) / 20
+    gbs = B * n * 4 * (2 * D + 6) / ms / 1e6
+    print(f"n {n} D {D} ms {ms:.4f} GB/s {gbs:.0f} frac {gbs / HBM:.3f}", flush=True)
