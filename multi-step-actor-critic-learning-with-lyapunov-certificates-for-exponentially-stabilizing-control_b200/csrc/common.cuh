@@ -77,6 +77,22 @@ inline bool row_store_misaligned(const void* p) {
   return p != nullptr && (reinterpret_cast<uintptr_t>(p) & mask) != 0;
 }
 
+// host-side checks shared by the rollout entry points `what`: the sampler path needs a time limit, and the env phase writes
+// the obs / obs2 / act rows of the transition record with store_row
+template <int ID>
+inline int check_rollout_outputs(const char* what, const msacl_env_state_t* st, const msacl_transitions_t* out) {
+  if (st->max_step <= 0) {
+    set_error("%s: the sampler path needs max_step > 0 (bare-env mode is msacl_env_step only)", what);
+    return MSACL_ERR_BAD_ARG;
+  }
+  if (row_store_misaligned<Env<ID>::D>(out->obs) || row_store_misaligned<Env<ID>::D>(out->obs2) || row_store_misaligned<Env<ID>::A>(out->act)) {
+    set_error("%s: transition obs/obs2/act rows must be aligned to their vector width (16 B if the row length is a multiple of 4 "
+              "floats, 8 B if even)", what);
+    return MSACL_ERR_BAD_ARG;
+  }
+  return MSACL_OK;
+}
+
 template <int ID>
 struct EnvRegs {
   using E = Env<ID>;

@@ -4,7 +4,7 @@
 // HBM-bound: algorithmic bytes per env-step = 4*(2*SF + 2*D + A + 1) + 8*2*SD + 2 + 32 (counters).
 #include <cstdarg>
 
-#include "common.cuh"
+#include "env_phase.cuh"
 
 namespace msacl {
 
@@ -90,90 +90,30 @@ env_step_kernel(msacl_env_state_t st, const float* __restrict__ action, float* _
 
 // One BaseSampler._n_step (RL/trainer/sampler/base.py:118-163,220) for policy outputs computed OUTSIDE the kernel: the
 // path for policies the fused rollout kernels are not specialised for (any depth / width / activation; the reference
-// builds arbitrary MLPs, RL/apprfunc/mlp.py:18-33).  Thread = env instance; same Philox streams, sampling arithmetic,
-// reward / cost scaling, autoreset and n-step run / emit bookkeeping as the env phase of rollout_fused.cu / rollout_tc.cu.
+// builds arbitrary MLPs, RL/apprfunc/mlp.py:18-33).  Thread = env instance; the env phase is the one of the fused
+// rollout kernels (env_phase.cuh).  The next observation is handed off through the env state, which the next step's first
+// layer reads: the state is stored in the hand-off, so its counters are dead before the transition stores (this keeps the
+// SingleTrackCar instance free of register spills).
 template <int ID>
 __global__ void __launch_bounds__(128)
 rollout_step_kernel(msacl_env_state_t st, const float* __restrict__ logits, float min_log_std, float max_log_std, uint32_t step,
                     int n_step, float reward_scale, float cost_scale, const float* __restrict__ eps, int deterministic,
                     msacl_transitions_t out, double* stats) {
-  using E = Env<ID>;
-  constexpr int D = E::D, A = E::A;
+  constexpr int A2 = 2 * Env<ID>::A;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  float v[5] = {0.f, 0.f, 0.f, 0.f, 0.f};      // episodes, sum of returns, sum of lengths, terminated, truncated
+  EpisodeStats epstats;
   if (i < st.n) {
     EnvRegs<ID> e;
     e.load(st, i);
-    float z[4] = {0.f, 0.f, 0.f, 0.f};
-    if (!deterministic) {
-      if (eps) {
+    float lg[A2];
 #pragma unroll
-        for (int j = 0; j < A; ++j) z[j] = eps[i * A + j];
-      } else {
-        action_noise4(st.seed, st.env_base + (uint64_t)i, step, z);
-      }
-    }
-    if (out.obs) store_row<D>(out.obs, i, e.obs());
-    float act[A];
-    float lp_gauss = 0.f, lp_tanh = 0.f, lp_scale = 0.f;
-#pragma unroll
-    for (int j = 0; j < A; ++j) {      // TanhGaussDistribution.sample / mode (act_distribution_cls.py:45-57, 90-95)
-      const float mean = logits[i * (2 * A) + j];
-      const float ls = logits[i * (2 * A) + A + j];
-      const float sd = expf(fminf(fmaxf(ls, min_log_std), max_log_std));
-      const float half = (E::act_high(j) - E::act_low(j)) / 2.0f;
-      const float mid = (E::act_high(j) + E::act_low(j)) / 2.0f;
-      const float u = deterministic ? mean : (sd * z[j] + mean);
-      const float th = tanhf(u);
-      const float a_lim = half * th + mid;
-      const float diff = u - mean;
-      const float g = ((-(diff * diff)) / (2.0f * (sd * sd)) - logf(sd)) - 0.91893853320467267f;
-      const float t = logf(1.000001f - th * th);
-      const float sc = logf(half);
-      lp_gauss = (j == 0) ? g : lp_gauss + g;
-      lp_tanh = (j == 0) ? t : lp_tanh + t;
-      lp_scale = (j == 0) ? sc : lp_scale + sc;
-      act[j] = fminf(fmaxf(a_lim, E::act_low(j)), E::act_high(j));       // base.py:141-143
-    }
-    const float logp = (lp_gauss - lp_tanh) - lp_scale;
-    const float rew = E::step(e.sf, e.sd, act);
-    const bool term = e.out_of_bounds();
-    e.step += 1;
-    const bool trunc = e.step >= st.max_step;
-    const bool done = term || trunc;
-    e.ep_return += rew;
-    e.ep_len += 1;
-    const float cost = np_rowsum_sq<D>(e.obs()) * cost_scale;          // rew_plus_cost.py:20-21 on real_next_obs
-    e.run = min(e.run + 1, n_step);
-    const bool emit = e.run >= n_step;
-    if (out.obs2) store_row<D>(out.obs2, i, e.obs());                  // pre-reset observation
-    if (done) {
-      v[0] = 1.f; v[1] = e.ep_return; v[2] = (float)e.ep_len;
-      if (term) v[3] = 1.f; else v[4] = 1.f;
-      e.episode += 1;
-      e.run = 0;
-      e.reset(st.seed, st.env_base + (uint64_t)i);
-    }
-    if (out.act) store_row<A>(out.act, i, act);
-    if (out.rew) out.rew[i] = rew * reward_scale;
-    if (out.cost) out.cost[i] = cost;
-    if (out.done) out.done[i] = done ? 1 : 0;
-    if (out.logp) out.logp[i] = logp;
-    if (out.emit) out.emit[i] = emit ? 1 : 0;
-    if (out.logits) {
-#pragma unroll
-      for (int j = 0; j < 2 * A; ++j) out.logits[i * (2 * A) + j] = logits[i * (2 * A) + j];
-    }
-    e.store(st, i);
+    for (int j = 0; j < A2; ++j) lg[j] = logits[i * A2 + j];
+    float z[4];
+    env_noise<Env<ID>::A>(z, !deterministic, eps, i, st.seed, st.env_base + (uint64_t)i, step);
+    env_phase<ID>(e, lg, z, deterministic, min_log_std, max_log_std, st, i, n_step, reward_scale, cost_scale, out, i, epstats,
+                  [&](const float*) { e.store(st, i); });
   }
-  if (stats) {                                   // one atomic per warp and statistic that saw an episode end
-#pragma unroll
-    for (int q = 0; q < 5; ++q) {
-#pragma unroll
-      for (int o = 16; o >= 1; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
-      if ((threadIdx.x & 31) == 0 && v[q] != 0.f) atomicAdd(&stats[q], (double)v[q]);
-    }
-  }
+  if (stats) epstats.flush(stats);
 }
 
 __global__ void action_noise_kernel(uint64_t seed, uint64_t env_base, int64_t n, int act_dim, uint32_t step, float* out) {
@@ -294,14 +234,10 @@ int msacl_rollout_step(const msacl_env_state_t* st, const float* logits, float m
                        const msacl_transitions_t* out, double* stats, void* stream) {
   if (int rc = validate_state(st)) return rc;
   if (!logits || !out || n_step <= 0) { set_error("rollout_step: bad argument"); return MSACL_ERR_BAD_ARG; }
-  if (st->max_step <= 0) { set_error("rollout_step: the sampler path needs max_step > 0 (bare-env mode is msacl_env_step only)"); return MSACL_ERR_BAD_ARG; }
   const int threads = 128;
   const unsigned blocks = (unsigned)((st->n + threads - 1) / threads);
   MSACL_DISPATCH_ENV(st->env_id, {
-    if (row_store_misaligned<Env<ID>::D>(out->obs) || row_store_misaligned<Env<ID>::D>(out->obs2) || row_store_misaligned<Env<ID>::A>(out->act)) {
-      set_error("rollout_step: transition obs/obs2/act rows must be aligned to their vector width (16 B if the row length is a multiple of 4 floats, 8 B if even)");
-      return MSACL_ERR_BAD_ARG;
-    }
+    if (int rc = check_rollout_outputs<ID>("rollout_step", st, out)) return rc;
     rollout_step_kernel<ID><<<blocks, threads, 0, (cudaStream_t)stream>>>(*st, logits, min_log_std, max_log_std, step, n_step, reward_scale,
                                                                           cost_scale, eps, deterministic, *out, stats);
   });

@@ -25,7 +25,8 @@
 //   * layer 3 (256 -> 2A) is applied to the layer-2 register tile and combined with a halving
 //     warp-shuffle reduction (62 shuffles / 64 values).
 // Compiled with -fmad=false: only the explicit __fmaf_rn calls below contract.
-#include "common.cuh"
+#include "env_phase.cuh"
+#include "tcgen05.cuh"
 
 namespace msacl {
 
@@ -59,37 +60,6 @@ struct Smem {
   unsigned long long full_bar[NSTAGE];
   unsigned long long empty_bar[NSTAGE];
 };
-
-// ---- mbarrier / TMA bulk-copy primitives (PTX ISA 8.x, sm_90+)
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(void* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(void* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(void* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(void* bar, uint32_t parity) {
-  const uint32_t a = smem_u32(bar);
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t"
-      "}" ::"r"(a), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, uint32_t bytes, void* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-
-__device__ __forceinline__ void bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-__device__ __forceinline__ void bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 // Halving butterfly: V values per lane summed over the 32 lanes; afterwards value
 // `orig` lives in v[0..V/32) of lane orig / (V/32) (V >= 32), or in v[0] of lanes
@@ -139,9 +109,9 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
   if (tid < 8) sm.b3[tid] = tid < A2 ? actor.b3[tid] : 0.f;
   if (tid == 0) {
 #pragma unroll
-    for (int i = 0; i < NSTAGE; ++i) { mbar_init(&sm.full_bar[i], 1); mbar_init(&sm.empty_bar[i], NGEMM / 32); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    for (int i = 0; i < NSTAGE; ++i) { tc::mbar_init(&sm.full_bar[i], 1); tc::mbar_init(&sm.empty_bar[i], NGEMM / 32); }
+    tc::mbar_fence_init();
+    tc::fence_async_smem();
   }
   __syncthreads();
 
@@ -159,9 +129,9 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
     auto produce = [&](int64_t gi) {          // issue chunk gi (global index) into stage gi % NSTAGE
       if (gi >= total_chunks) return;
       const int stg = (int)(gi % NSTAGE);
-      if (gi >= NSTAGE) mbar_wait(&sm.empty_bar[stg], (uint32_t)(((gi / NSTAGE) & 1) ^ 1));
-      mbar_expect_tx(&sm.full_bar[stg], CHUNK_BYTES);
-      tma_bulk_g2s(sm.wc[stg], actor.w2t + (size_t)(gi % NCHUNK) * KC * HID, CHUNK_BYTES, &sm.full_bar[stg]);
+      if (gi >= NSTAGE) tc::mbar_wait(&sm.empty_bar[stg], (uint32_t)(((gi / NSTAGE) & 1) ^ 1));
+      tc::mbar_expect_tx(&sm.full_bar[stg], CHUNK_BYTES);
+      tc::tma_bulk_g2s(sm.wc[stg], actor.w2t + (size_t)(gi % NCHUNK) * KC * HID, CHUNK_BYTES, &sm.full_bar[stg]);
     };
     if (producer) {
 #pragma unroll
@@ -173,7 +143,7 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
       const int nt = (int)((num_tiles - NTILE * pair) < NTILE ? (num_tiles - NTILE * pair) : NTILE);
       for (int k = 0; k < K; ++k) {
         for (int T = 0; T < nt; ++T) {
-          bar_sync(BAR_XREADY + T, NGEMM + TM);   // obs tile T is in smem
+          tc::bar_sync(BAR_XREADY + T, NGEMM + TM);   // obs tile T is in smem
           float acc[8][8];
           // ---- layer 1 on the same thread tile as layer 2 (envs m0..m0+8 x 8 units)
           {
@@ -224,7 +194,7 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
           for (int ch = 0; ch < NCHUNK; ++ch, ++g) {
             if (producer) produce(g + PREFETCH);
             const int stg = (int)(g % NSTAGE);
-            mbar_wait(&sm.full_bar[stg], (uint32_t)((g / NSTAGE) & 1));
+            tc::mbar_wait(&sm.full_bar[stg], (uint32_t)((g / NSTAGE) & 1));
             const float* wb = sm.wc[stg] + lane * 4;
             // swizzle key of hidden unit kg = ch*16 + kk is (kg>>2)&7 = ((ch&1)<<2) | (kk>>2):
             // pair index = warp ^ (key>>1) (runtime, per 8 k's), order inside the pair = key&1 (compile time)
@@ -249,7 +219,7 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
               }
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive(&sm.empty_bar[stg]);   // this warp is done with the stage
+            if (lane == 0) tc::mbar_arrive(&sm.empty_bar[stg]);   // this warp is done with the stage
           }
 
           // ---- bias + ReLU, then layer 3 on the register tile
@@ -297,7 +267,7 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
             }
           }
           __threadfence_block();
-          bar_arrive(BAR_LOGITS + T, NGEMM + TM);   // logits of tile T are in smem
+          tc::bar_arrive(BAR_LOGITS + T, NGEMM + TM);   // logits of tile T are in smem
         }
       }
     }
@@ -305,7 +275,7 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
     // =========================== env warps ===========================
     const int T = (tid - NGEMM) >> 6;        // tile slot owned by this warp pair
     const int et = (tid - NGEMM) & (TM - 1); // env within the tile
-    float st_ep = 0.f, st_ret = 0.f, st_len = 0.f, st_term = 0.f, st_trunc = 0.f;
+    EpisodeStats epstats;
     for (int64_t pair = blockIdx.x; pair < num_pairs; pair += gridDim.x) {
       const int64_t tile = NTILE * pair + T;
       if (tile >= num_tiles) break;          // CTA-uniform per warp pair; GEMM warps skip this slot too
@@ -321,101 +291,30 @@ rollout_fused_kernel(msacl_env_state_t st, msacl_actor_t actor, int K, uint32_t 
         for (int d = 0; d < D; ++d) sm.x[T][d * TM + et] = 0.f;
       }
       __threadfence_block();
-      bar_arrive(BAR_XREADY + T, NGEMM + TM);
+      tc::bar_arrive(BAR_XREADY + T, NGEMM + TM);
       for (int k = 0; k < K; ++k) {
-        bar_sync(BAR_LOGITS + T, NGEMM + TM);
+        tc::bar_sync(BAR_LOGITS + T, NGEMM + TM);
         if (owner) {
           const int64_t row = (int64_t)k * st.n + gi;
-          if (out.obs) {
-            store_row<D>(out.obs, row, r.obs());
-          }
-          float z[4] = {0.f, 0.f, 0.f, 0.f};
-          if (!deterministic) {
-            if (eps) {
+          float z[4];
+          env_noise<A>(z, !deterministic, eps, row, st.seed, st.env_base + (uint64_t)gi, step_base + (uint32_t)k);
+          float lg[A2];
 #pragma unroll
-              for (int j = 0; j < A; ++j) z[j] = eps[row * A + j];
-            } else {
-              action_noise4(st.seed, st.env_base + (uint64_t)gi, step_base + (uint32_t)k, z);
-            }
-          }
-          float act[A];
-          float lp_gauss = 0.f, lp_tanh = 0.f, lp_scale = 0.f;
+          for (int j = 0; j < A2; ++j) lg[j] = sm.out[T][j * TM + et];
+          env_phase<ID>(r, lg, z, deterministic, actor.min_log_std, actor.max_log_std, st, gi, n_step, reward_scale, cost_scale,
+                        out, row, epstats, [&](const float* obs) {
 #pragma unroll
-          for (int j = 0; j < A; ++j) {
-            const float mean = sm.out[T][j * TM + et];
-            const float ls = sm.out[T][(A + j) * TM + et];
-            const float sd = expf(fminf(fmaxf(ls, actor.min_log_std), actor.max_log_std));
-            const float half = (E::act_high(j) - E::act_low(j)) / 2.0f;
-            const float mid = (E::act_high(j) + E::act_low(j)) / 2.0f;
-            const float u = deterministic ? mean : (sd * z[j] + mean);      // torch.normal: z*std, then +mean
-            const float th = tanhf(u);
-            const float a_lim = half * th + mid;
-            // Normal.log_prob(u) = -((u-mean)^2)/(2 var) - log(std) - log(sqrt(2 pi))
-            const float diff = u - mean;
-            const float g = ((-(diff * diff)) / (2.0f * (sd * sd)) - logf(sd)) - 0.91893853320467267f;
-            const float t = logf(1.000001f - th * th);
-            const float sc = logf(half);
-            lp_gauss = (j == 0) ? g : lp_gauss + g;
-            lp_tanh = (j == 0) ? t : lp_tanh + t;
-            lp_scale = (j == 0) ? sc : lp_scale + sc;
-            act[j] = fminf(fmaxf(a_lim, E::act_low(j)), E::act_high(j));   // base.py:141-143
-          }
-          const float logp = (lp_gauss - lp_tanh) - lp_scale;
-
-          const float rew = E::step(r.sf, r.sd, act);
-          const bool term = r.out_of_bounds();
-          r.step += 1;
-          const bool trunc = r.step >= st.max_step;
-          const bool done = term || trunc;
-          r.ep_return += rew;
-          r.ep_len += 1;
-          const float rew_s = rew * reward_scale;                                  // rew_plus_cost.py:18
-          const float cost = np_rowsum_sq<D>(r.obs()) * cost_scale;                // :20-21
-          r.run = min(r.run + 1, n_step);
-          const bool emit = r.run >= n_step;
-          if (out.act) {
-            store_row<A>(out.act, row, act);
-          }
-          if (out.obs2) {
-            store_row<D>(out.obs2, row, r.obs());                                  // real_next_obs (pre-reset)
-          }
-          if (out.rew) out.rew[row] = rew_s;
-          if (out.cost) out.cost[row] = cost;
-          if (out.done) out.done[row] = done ? 1 : 0;
-          if (out.logp) out.logp[row] = logp;
-          if (out.emit) out.emit[row] = emit ? 1 : 0;
-          if (out.logits) {
-#pragma unroll
-            for (int j = 0; j < 2 * A; ++j) out.logits[row * (2 * A) + j] = sm.out[T][j * TM + et];
-          }
-          if (done) {      // episode statistics: per-thread partials, reduced once per launch (no hot atomics)
-            st_ep += 1.f; st_ret += r.ep_return; st_len += (float)r.ep_len;
-            if (term) st_term += 1.f; else st_trunc += 1.f;
-          }
-          if (done) {
-            r.episode += 1;
-            r.run = 0;
-            r.reset(st.seed, st.env_base + (uint64_t)gi);
-          }
-#pragma unroll
-          for (int d = 0; d < D; ++d) sm.x[T][d * TM + et] = r.obs()[d];
+            for (int d = 0; d < D; ++d) sm.x[T][d * TM + et] = obs[d];
+          });
         }
         if (k + 1 < K) {
           __threadfence_block();
-          bar_arrive(BAR_XREADY + T, NGEMM + TM);
+          tc::bar_arrive(BAR_XREADY + T, NGEMM + TM);
         }
       }
       if (owner) r.store(st, gi);
     }
-    if (stats) {
-      float v[5] = {st_ep, st_ret, st_len, st_term, st_trunc};
-#pragma unroll
-      for (int q = 0; q < 5; ++q) {
-#pragma unroll
-        for (int o = 16; o >= 1; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
-        if (lane == 0 && v[q] != 0.f) atomicAdd(&stats[q], (double)v[q]);
-      }
-    }
+    if (stats) epstats.flush(stats);
   }
 }
 
@@ -428,16 +327,12 @@ extern "C" int msacl_rollout_fused(const msacl_env_state_t* st, const msacl_acto
                                    const float* eps, int32_t deterministic, const msacl_transitions_t* out,
                                    double* stats, void* stream) {
   if (!st || !actor || !out || st->n <= 0 || K <= 0 || n_step <= 0) { set_error("rollout_fused: bad argument"); return MSACL_ERR_BAD_ARG; }
-  if (st->max_step <= 0) { set_error("rollout_fused: the sampler path needs max_step > 0 (bare-env mode is msacl_env_step only)"); return MSACL_ERR_BAD_ARG; }
   if (!actor->w1 || !actor->b1 || !actor->w2t || !actor->b2 || !actor->w3 || !actor->b3) { set_error("rollout_fused: null actor weights"); return MSACL_ERR_BAD_ARG; }
   if ((reinterpret_cast<uintptr_t>(actor->w2t) & 15) != 0) { set_error("rollout_fused: w2t must be 16-byte aligned"); return MSACL_ERR_BAD_ARG; }
   const int64_t pairs = ((st->n + TM - 1) / TM + NTILE - 1) / NTILE;
   const unsigned grid = (unsigned)(pairs < kNumSMs ? pairs : kNumSMs);
   MSACL_DISPATCH_ENV(st->env_id, {
-    if (row_store_misaligned<Env<ID>::D>(out->obs) || row_store_misaligned<Env<ID>::D>(out->obs2) || row_store_misaligned<Env<ID>::A>(out->act)) {
-      set_error("rollout_fused: transition obs/obs2/act rows must be aligned to their vector width (16 B if the row length is a multiple of 4 floats, 8 B if even)");
-      return MSACL_ERR_BAD_ARG;
-    }
+    if (int rc = check_rollout_outputs<ID>("rollout_fused", st, out)) return rc;
     const size_t smem = sizeof(Smem<ID>);
     auto kern = rollout_fused_kernel<ID>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

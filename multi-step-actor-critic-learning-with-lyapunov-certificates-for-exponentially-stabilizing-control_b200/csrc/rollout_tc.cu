@@ -25,7 +25,7 @@
 // logits); tcgen05.commit signals the ones the tensor pipe produces.
 // The alternatives measured against this layout (two tiles per env warpgroup, a dedicated epilogue-1 group, 2 or 4 tile
 // slots) are in DESIGN.md §4.1.
-#include "common.cuh"
+#include "env_phase.cuh"
 #include "tcgen05.cuh"
 
 namespace msacl {
@@ -270,7 +270,7 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
     const int w = warp >> 2;                 // env warpgroup: tile slots w, w + NS, ...
     const int r = tid & (TCM - 1);
     uint32_t lcount = 0;                     // logits deliveries each of its tile slots has consumed
-    float st_ep = 0.f, st_ret = 0.f, st_len = 0.f, st_term = 0.f, st_trunc = 0.f;
+    EpisodeStats epstats;
     auto write_xop = [&](const float* obs, bool valid) {
       float v[16];
 #pragma unroll
@@ -306,16 +306,10 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         for (int s = w; s < nt; s += NS) {
         const int64_t gi = (tile0 + s) * TCM + r;
         const bool owner = gi < st.n;
+        const int64_t row = (int64_t)k * st.n + gi;
         // the action noise of this step does not depend on the logits: draw it while the tile's MLP is still running
-        float z[4] = {0.f, 0.f, 0.f, 0.f};
-        if (owner && !deterministic) {
-          if (eps) {
-#pragma unroll
-            for (int j = 0; j < A; ++j) z[j] = eps[((int64_t)k * st.n + gi) * A + j];
-          } else {
-            action_noise4(st.seed, st.env_base + (uint64_t)gi, step_base + (uint32_t)k, z);
-          }
-        }
+        float z[4];
+        env_noise<A>(z, owner && !deterministic, eps, row, st.seed, st.env_base + (uint64_t)gi, step_base + (uint32_t)k);
 #ifdef MSACL_TC_TIMING
         const long long t_w0 = clock64();
 #endif
@@ -326,77 +320,13 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
         float lg[A2];
 #pragma unroll
         for (int j = 0; j < A2; ++j) lg[j] = logits_of(s)[j * TCM + r];
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + w) : "memory");
+        tc::bar_sync(1 + w, 128);
 #ifdef MSACL_TC_TIMING
         const long long t_w1 = clock64();
 #endif
         if (owner) {
-          const int64_t row = (int64_t)k * st.n + gi;
-          if (out.obs) {
-            store_row<D>(out.obs, row, e.obs());
-          }
-          if (out.logits) {      // diagnostic output, written here so that the logits do not stay live across the env step
-#pragma unroll
-            for (int j = 0; j < A2; ++j) out.logits[row * A2 + j] = lg[j];
-          }
-          float act[A];
-          float lp_gauss = 0.f, lp_tanh = 0.f, lp_scale = 0.f;
-#pragma unroll
-          for (int j = 0; j < A; ++j) {
-            const float mean = lg[j];
-            const float ls = lg[A + j];
-            const float sd = expf(fminf(fmaxf(ls, actor.min_log_std), actor.max_log_std));
-            const float half = (E::act_high(j) - E::act_low(j)) / 2.0f;
-            const float mid = (E::act_high(j) + E::act_low(j)) / 2.0f;
-            const float u = deterministic ? mean : (sd * z[j] + mean);
-            const float th = tanhf(u);
-            const float a_lim = half * th + mid;
-            const float diff = u - mean;
-            const float g = ((-(diff * diff)) / (2.0f * (sd * sd)) - logf(sd)) - 0.91893853320467267f;
-            const float t = logf(1.000001f - th * th);
-            const float sc = logf(half);
-            lp_gauss = (j == 0) ? g : lp_gauss + g;
-            lp_tanh = (j == 0) ? t : lp_tanh + t;
-            lp_scale = (j == 0) ? sc : lp_scale + sc;
-            act[j] = fminf(fmaxf(a_lim, E::act_low(j)), E::act_high(j));
-          }
-          const float logp = (lp_gauss - lp_tanh) - lp_scale;
-          const float rew = E::step(e.sf, e.sd, act);
-          const bool term = e.out_of_bounds();
-          e.step += 1;
-          const bool trunc = e.step >= st.max_step;
-          const bool done = term || trunc;
-          e.ep_return += rew;
-          e.ep_len += 1;
-          const float rew_s = rew * reward_scale;
-          const float cost = np_rowsum_sq<D>(e.obs()) * cost_scale;
-          e.run = min(e.run + 1, n_step);
-          const bool emit = e.run >= n_step;
-          float obs2[D];                                  // real_next_obs (pre-reset)
-#pragma unroll
-          for (int d = 0; d < D; ++d) obs2[d] = e.obs()[d];
-          if (done) {      // episode statistics: per-thread partials, reduced once per launch (no hot atomics)
-            st_ep += 1.f; st_ret += e.ep_return; st_len += (float)e.ep_len;
-            if (term) st_term += 1.f; else st_trunc += 1.f;
-            e.episode += 1;
-            e.run = 0;
-            e.reset(st.seed, st.env_base + (uint64_t)gi);
-          }
-          // hand the next observation to the tensor pipeline FIRST: the proxy fence inside write_xop
-          // waits for this thread's outstanding memory operations, so the (uncoalesced) transition
-          // stores are issued after it and drain while the MLP of this tile is already running
-          if (k + 1 < K) write_xop(e.obs(), true);
-          if (out.act) {
-            store_row<A>(out.act, row, act);
-          }
-          if (out.obs2) {
-            store_row<D>(out.obs2, row, obs2);
-          }
-          if (out.rew) out.rew[row] = rew_s;
-          if (out.cost) out.cost[row] = cost;
-          if (out.done) out.done[row] = done ? 1 : 0;
-          if (out.logp) out.logp[row] = logp;
-          if (out.emit) out.emit[row] = emit ? 1 : 0;
+          env_phase<ID>(e, lg, z, deterministic, actor.min_log_std, actor.max_log_std, st, gi, n_step, reward_scale, cost_scale,
+                        out, row, epstats, [&](const float* obs) { if (k + 1 < K) write_xop(obs, true); });
         } else if (k + 1 < K) {
           write_xop(e.obs(), false);
         }
@@ -414,15 +344,7 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
       const int64_t gi = (tile0 + w) * TCM + r;
       if (gi < st.n) e.store(st, gi);
     }
-    if (stats) {
-      float v[5] = {st_ep, st_ret, st_len, st_term, st_trunc};
-#pragma unroll
-      for (int q = 0; q < 5; ++q) {
-#pragma unroll
-        for (int o = 16; o >= 1; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
-        if (lane == 0 && v[q] != 0.f) atomicAdd(&stats[q], (double)v[q]);
-      }
-    }
+    if (stats) epstats.flush(stats);
   } else if (warp < W_MMA) {
     // =========================== epilogue warps (8): both epilogues, column-split ===========================
     // Warp e = warp - W_EPI1: TMEM lane quadrant q = e & 3 (rows 32q..32q+31, thread = row), column half h = e >> 2.
@@ -524,7 +446,7 @@ rollout_tc_kernel(msacl_env_state_t st, msacl_actor_t actor, const unsigned char
           part[(2 * p + 1) * TCM + r] = hi;
         }
       }
-      asm volatile("bar.sync %0, 64;" ::"r"(4 + q) : "memory");
+      tc::bar_sync(4 + q, 64);
       if (h == 0) {
 #pragma unroll
         for (int p = 0; p < NP; ++p) {
@@ -711,14 +633,10 @@ extern "C" int msacl_rollout_fused_tc(const msacl_env_state_t* st, const msacl_a
                                       float cost_scale, const float* eps, int32_t deterministic,
                                       const msacl_transitions_t* out, double* stats, void* stream) {
   if (!st || !actor || !out || !w1p || !w2p || st->n <= 0 || K <= 0 || n_step <= 0) { set_error("rollout_fused_tc: bad argument"); return MSACL_ERR_BAD_ARG; }
-  if (st->max_step <= 0) { set_error("rollout_fused_tc: the sampler path needs max_step > 0 (bare-env mode is msacl_env_step only)"); return MSACL_ERR_BAD_ARG; }
   if ((reinterpret_cast<uintptr_t>(w2p) & 15) || (reinterpret_cast<uintptr_t>(w1p) & 15)) { set_error("rollout_fused_tc: packed weights must be 16-byte aligned"); return MSACL_ERR_BAD_ARG; }
   const int64_t tiles = (st->n + TCM - 1) / TCM;
   MSACL_DISPATCH_ENV(st->env_id, {
-    if (row_store_misaligned<Env<ID>::D>(out->obs) || row_store_misaligned<Env<ID>::D>(out->obs2) || row_store_misaligned<Env<ID>::A>(out->act)) {
-      set_error("rollout_fused_tc: transition obs/obs2/act rows must be aligned to their vector width (16 B if the row length is a multiple of 4 floats, 8 B if even)");
-      return MSACL_ERR_BAD_ARG;
-    }
+    if (int rc = check_rollout_outputs<ID>("rollout_fused_tc", st, out)) return rc;
     static_assert(sizeof(TcSmem<ID>) + 128 <= 232448, "shared-memory layout exceeds the 227 KB per-CTA limit");
     const int64_t cap = g_tc_max_ctas > 0 ? g_tc_max_ctas : kNumSMs;
     const unsigned grid = (unsigned)(tiles < cap ? tiles : cap);      // balanced shares: every CTA owns >= 1 tile

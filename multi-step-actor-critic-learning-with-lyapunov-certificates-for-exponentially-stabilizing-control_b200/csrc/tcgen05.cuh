@@ -1,4 +1,4 @@
-// Minimal tcgen05 / TMEM / mbarrier / TMA-bulk primitives for sm_100a (inline PTX).
+// Minimal tcgen05 / TMEM / mbarrier / TMA-bulk / named-barrier primitives for sm_100a (inline PTX).
 //
 // Shared-memory operand layout used throughout (UMMA "K-major, SWIZZLE_NONE / interleave"
 // canonical form, see cute/arch/mma_sm100_desc.hpp and cute/atom/mma_traits_sm100.hpp in the
@@ -76,6 +76,10 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, uint32_
 
 // generic-proxy writes to shared memory -> visible to the async proxy (UMMA operand reads)
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+// ---- named barriers (`count` threads, a multiple of 32)
+__device__ __forceinline__ void bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
+__device__ __forceinline__ void bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 // ---- TMEM
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {   // one full warp
