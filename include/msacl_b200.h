@@ -377,7 +377,8 @@ int msacl_adam_tick(int32_t* step, float* dyn, double lr, double beta1, double b
  * mode 3: FP64 DFMA throughput at full occupancy;
  * modes 4-6: separate DMUL / DADD issued by ONE warp per SM sub-partition with 8 / 2 / 1 independent chains per thread
  *         (*flops then returns the FP64 instructions issued per warp): the FP64 issue rate the fused rollout's env phase sees;
- * mode 7: float32 <-> float64 round trips (two conversions + one DMUL each; *flops = round trips per warp).
+ * mode 7: float32 <-> float64 round trips (two conversions + one DMUL each; *flops = round trips per warp);
+ * mode 8: the mode-1 outer product with directed rounding (half FFMA.RM, half FFMA.RP), the interval GEMM ceiling.
  * sink: device float[128] (sink[64..128) is read as operand source in mode 1).
  * Returns the FLOPs issued in *flops (host). */
 int msacl_ffma_probe(int32_t mode, int32_t iters, float* sink, double* flops, void* stream);
@@ -465,6 +466,109 @@ int msacl_certify_steps(int64_t n, int32_t obs_dim, int32_t K, int32_t k0, const
 int msacl_certify_finish(int64_t n, int32_t horizon, const msacl_cert_records_t* rec, int64_t* summary, void* stream);
 /* summary[MSACL_CERT_SUM_ROA] = #{i < n : v0[i] < c_star} (zeroed by the call). */
 int msacl_certify_roa(int64_t n, const float* v0, float c_star, int64_t* summary, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Region verifier of the Lyapunov certificate (no counterpart in the reference): interval branch-and-bound over state boxes.
+ * For a box X0, an inner box B, eta, alpha1, alpha2 and m >= 1 closed-loop steps it partitions X0 \ B into dyadic cells and
+ * proves per cell C, with outward-rounded interval arithmetic:
+ *   DECREASE ok  sup V(F^m(C)) <= (1 - eta)^m inf V(C)
+ *   ESCAPED ok   F^j(C) lies strictly inside the env's observation bounds for j = 1..m (the env cannot terminate)
+ *   BOUND ok     alpha1 sup |x|^2 <= inf V(C) and sup V(C) <= alpha2 inf |x|^2 over C
+ *   NONFINITE    some bound overflowed or is NaN; such a cell is never verified
+ * F is one greedy closed-loop step: policy mean mu, a = half tanh(mu) + mid, clip to the action box, CONTROL_STEP
+ * explicit-Euler sub-steps.  The verified object is the REAL-ARITHMETIC closed loop: the networks as exact real functions of
+ * their stored float32 parameters, exact sin / cos / tanh, the Euler map in exact arithmetic (the env's constants read as
+ * exact reals).  The rounding of any float implementation (split-bf16 rollout GEMMs, float32 env kernels) is not modelled.
+ * Envs: VanderPol, Pendulum, DuctedFan, TwoLink.
+ * --------------------------------------------------------------------------------------------------------------- */
+enum {
+  MSACL_REGION_NONFINITE = 1,         /* cell flags (msacl_region_out_t.flags) */
+  MSACL_REGION_DECREASE = 2,          /* DECREASE not proven */
+  MSACL_REGION_ESCAPED = 4,           /* ESCAPED not proven */
+  MSACL_REGION_BOUND = 8,             /* BOUND not proven */
+  MSACL_REGION_LEAVES = 16,           /* F^m(C) not proven inside X0 */
+  MSACL_REGION_REFUTE_DECREASE = 32,  /* proven: inf V(F^m(C)) > (1 - eta)^m sup V(C), i.e. every point of C violates DECREASE */
+  MSACL_REGION_REFUTE_ESCAPED = 64,   /* proven: some F^j(C), j <= m, lies entirely outside the observation bounds */
+  MSACL_REGION_HIDDEN = 256,          /* network width of the kernels (narrower layers are zero-padded) */
+  MSACL_REGION_MAX_DEPTH = 50
+};
+
+/* cell status written by msacl_region_round (msacl_region_ws_t.status) */
+enum { MSACL_REGION_SPLIT = 0, MSACL_REGION_VERIFIED = 1, MSACL_REGION_REFUTED = 2, MSACL_REGION_UNDECIDED = 3, MSACL_REGION_INNER = 4 };
+
+/* int64 statistics accumulated by msacl_region_round; volumes in units of 2^-50 of X0; keys are order keys of float32
+ * (MSACL_CERT_SUM_CSTAR_KEY): C_SOUND min (init +inf), C_IN / V_INNER max (init -inf) */
+enum {
+  MSACL_REGION_ST_VERIFIED = 0, MSACL_REGION_ST_REFUTED = 1, MSACL_REGION_ST_UNDECIDED = 2, MSACL_REGION_ST_INNER = 3,
+  MSACL_REGION_ST_SPLIT = 4, MSACL_REGION_ST_EVALUATED = 5, MSACL_REGION_ST_PROBED = 6,
+  MSACL_REGION_ST_FLAGS = 7,          /* [7 + b]: non-inner leaf cells with flag bit b (NONFINITE .. LEAVES) */
+  MSACL_REGION_ST_VOLUME = 12,        /* [12 + s]: volume of VERIFIED, REFUTED, UNDECIDED, INNER leaves */
+  MSACL_REGION_ST_C_SOUND = 16,       /* min inf V(C) over non-inner leaves that are not verified or whose F^m(C) may leave X0 */
+  MSACL_REGION_ST_C_IN = 17,          /* max sup V(F^m(C)) over inner leaves */
+  MSACL_REGION_ST_V_INNER = 18,       /* max sup V(C) over inner leaves */
+  MSACL_REGION_ST_INNER_FAIL = 19,    /* inner leaves that are NONFINITE, ESCAPED or LEAVES */
+  MSACL_REGION_ST_COUNT = 20
+};
+
+typedef struct {
+  int32_t env_id, obs_dim, act_dim;
+  int32_t p_h1, p_h2;                 /* policy obs -> p_h1 -> p_h2 -> 2 act_dim, ReLU, torch Linear layout [out][in] */
+  const float *p_w1, *p_b1, *p_w2, *p_b2, *p_w3, *p_b3;
+  int32_t v_h1, v_h2, v_out;          /* V net obs -> v_h1 -> v_h2 -> v_out (<= 256 each), V = sum z^2 */
+  const float *v_w1, *v_b1, *v_w2, *v_b2, *v_w3, *v_b3;
+} msacl_region_nets_t;
+
+typedef struct {
+  int32_t env_id, steps;              /* m >= 1 */
+  int32_t v_tanh;                     /* V hidden activation: 0 ReLU, 1 tanh */
+  double decay_lo, decay_hi;          /* (1 - eta)^m rounded down / up */
+  double alpha1, alpha2;
+  float x0_lo[16], x0_hi[16];         /* X0 */
+} msacl_region_params_t;
+
+typedef struct {                      /* per cell outputs of msacl_region_eval, [n] unless noted */
+  float *v_lo, *v_hi;                 /* inf / sup V(C) */
+  float *vm_lo, *vm_hi;               /* inf / sup V(F^m(C)) */
+  float *img_lo, *img_hi;             /* [n][obs_dim] box of F^m(C) */
+  uint8_t* flags;                     /* MSACL_REGION_* cell flags */
+  float* margin;                      /* proven violation of a REFUTE flag (decrease first), else 0 */
+  float* trace;                       /* optional [n][steps][4 act_dim + 2 obs_dim]: mu lo, mu hi, a lo, a hi, F^j lo, F^j hi */
+} msacl_region_out_t;
+
+typedef struct {
+  int32_t max_depth;                  /* 1..MSACL_REGION_MAX_DEPTH; depth t bisects dimension t mod obs_dim */
+  int32_t inner_level;                /* B is snapped outward to the grid of 2^inner_level cells per dimension */
+  uint32_t inner_lo[16], inner_hi[16];/* B = X0_lo + (X0_hi - X0_lo) [inner_lo, inner_hi] / 2^inner_level per dimension */
+  double inner_box_lo[16], inner_box_hi[16];   /* the snapped B in coordinates, rounded outward */
+  int64_t max_examples;               /* capacity of the counterexample list */
+} msacl_region_bnb_t;
+
+typedef struct {                      /* scratch of one msacl_region_round for k cells (device arrays) */
+  uint32_t* cells;                    /* [k][1 + obs_dim] copy of the popped cells */
+  float *lo, *hi;                     /* [k][obs_dim] their boxes */
+  msacl_region_out_t res;             /* [k] their evaluation (trace unused) */
+  float *plo, *phi;                   /* [k][obs_dim] centres probed for refutation */
+  msacl_region_out_t pres;            /* [k] evaluation of the centres */
+  int32_t* probe;                     /* [k] probe slot of cell i, -1 if none */
+  uint8_t* status;                    /* [k] MSACL_REGION_SPLIT .. INNER */
+  int64_t* scan;                      /* [3 * (k / 256 + 1) + 8] */
+} msacl_region_ws_t;
+
+/* Bytes of the packed network image (floats, 16-byte aligned). */
+int64_t msacl_region_image_bytes(void);
+/* Pack the policy and V net into the image: zero-padded to 256 units, the 256-wide matrices as [k][W+ | W-] rows. */
+int msacl_region_pack(const msacl_region_nets_t* nets, float* image, void* stream);
+/* Enclose F, V and the cell conditions for the n boxes [lo, hi] ([n][obs_dim], float32); n is *n_dev when n_dev != NULL
+ * (n is then an upper bound).  One persistent CTA per SM, FP32 FFMA.RM / FFMA.RP interval GEMMs. */
+int msacl_region_eval(const msacl_region_params_t* p, const float* image, int64_t n, const int64_t* n_dev, const float* lo,
+                      const float* hi, const msacl_region_out_t* out, void* stream);
+/* One branch-and-bound round over the k cells stack[top - k, top) (cell = [depth, idx_0 .. idx_{obs_dim-1}] uint32):
+ * evaluate, probe the centres of failing cells outside B for a proven counterexample, classify, accumulate stats, append up to
+ * max_examples counterexamples ([obs_dim centre, margin, kind 1 = decrease / 2 = escaped] floats) in a deterministic order,
+ * and write the children of split cells to stack[top - k, ...); *children (device) = their number. */
+int msacl_region_round(const msacl_region_params_t* p, const msacl_region_bnb_t* b, const float* image, uint32_t* stack,
+                       int64_t top, int64_t k, const msacl_region_ws_t* ws, int64_t* stats, float* examples, int64_t* children,
+                       void* stream);
 
 const char* msacl_last_error(void);
 int msacl_abi_version(void);

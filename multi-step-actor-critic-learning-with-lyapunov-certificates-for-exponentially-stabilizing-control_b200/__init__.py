@@ -6,7 +6,7 @@ upstream project; `msacl_b200.py` at the repo root aliases it).
 from .specs import ENV_NAMES, SPECS, get_spec  # noqa: F401
 
 __all__ = ["ENV_NAMES", "SPECS", "get_spec", "create_envs", "create_sampler", "create_buffer", "create_alg", "create_evaluator",
-           "create_trainer", "create_certifier", "load_library"]
+           "create_trainer", "create_certifier", "create_region_certifier", "load_library"]
 
 
 def load_library():
@@ -72,3 +72,12 @@ def create_certifier(**kwargs):
     the sampled states and horizon, not a proof.  `create_certifier(networks=..., env_name=..., num_states=N).run()`."""
     from .certify import B200CertificateVerifier
     return B200CertificateVerifier(**kwargs)
+
+
+def create_region_certifier(**kwargs):
+    """Sound region verifier of the Lyapunov certificate (no counterpart in the reference): interval branch-and-bound over
+    the cells of a state box X0 \\ B, proving V's (1 - eta)^m decrease over m greedy closed-loop steps for every state of a
+    verified cell, for the real-arithmetic closed loop.  `create_region_certifier(networks=..., env_name=..., box=(lo, hi),
+    inner=r).run()` -> RegionReport."""
+    from .certify_region import B200RegionVerifier
+    return B200RegionVerifier(**kwargs)

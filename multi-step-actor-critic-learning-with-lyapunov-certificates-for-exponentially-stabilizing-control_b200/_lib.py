@@ -58,6 +58,34 @@ class CertRecords(C.Structure):
                 ("worst_ratio", vp)]
 
 
+class RegionNets(C.Structure):
+    _fields_ = [("env_id", C.c_int32), ("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("p_h1", C.c_int32), ("p_h2", C.c_int32),
+                ("p_w1", vp), ("p_b1", vp), ("p_w2", vp), ("p_b2", vp), ("p_w3", vp), ("p_b3", vp),
+                ("v_h1", C.c_int32), ("v_h2", C.c_int32), ("v_out", C.c_int32),
+                ("v_w1", vp), ("v_b1", vp), ("v_w2", vp), ("v_b2", vp), ("v_w3", vp), ("v_b3", vp)]
+
+
+class RegionParams(C.Structure):
+    _fields_ = [("env_id", C.c_int32), ("steps", C.c_int32), ("v_tanh", C.c_int32), ("decay_lo", C.c_double),
+                ("decay_hi", C.c_double), ("alpha1", C.c_double), ("alpha2", C.c_double), ("x0_lo", C.c_float * 16),
+                ("x0_hi", C.c_float * 16)]
+
+
+class RegionOut(C.Structure):
+    _fields_ = [("v_lo", vp), ("v_hi", vp), ("vm_lo", vp), ("vm_hi", vp), ("img_lo", vp), ("img_hi", vp), ("flags", vp),
+                ("margin", vp), ("trace", vp)]
+
+
+class RegionBnb(C.Structure):
+    _fields_ = [("max_depth", C.c_int32), ("inner_level", C.c_int32), ("inner_lo", C.c_uint32 * 16), ("inner_hi", C.c_uint32 * 16),
+                ("inner_box_lo", C.c_double * 16), ("inner_box_hi", C.c_double * 16), ("max_examples", C.c_int64)]
+
+
+class RegionWs(C.Structure):
+    _fields_ = [("cells", vp), ("lo", vp), ("hi", vp), ("res", RegionOut), ("plo", vp), ("phi", vp), ("pres", RegionOut),
+                ("probe", vp), ("status", vp), ("scan", vp)]
+
+
 f32 = C.c_float
 i32, i64 = C.c_int32, C.c_int64
 
@@ -122,6 +150,11 @@ SIGNATURES = {
     "msacl_certify_steps": (C.c_int, [i64, i32, i32, i32, vp, vp, vp, C.POINTER(CertParams), C.POINTER(CertRecords), vp]),
     "msacl_certify_finish": (C.c_int, [i64, i32, C.POINTER(CertRecords), vp, vp]),
     "msacl_certify_roa": (C.c_int, [i64, vp, f32, vp, vp]),
+    "msacl_region_image_bytes": (C.c_int64, []),
+    "msacl_region_pack": (C.c_int, [C.POINTER(RegionNets), vp, vp]),
+    "msacl_region_eval": (C.c_int, [C.POINTER(RegionParams), vp, i64, vp, vp, vp, C.POINTER(RegionOut), vp]),
+    "msacl_region_round": (C.c_int, [C.POINTER(RegionParams), C.POINTER(RegionBnb), vp, vp, i64, i64, C.POINTER(RegionWs), vp, vp,
+                                     vp, vp]),
 }
 
 

@@ -21,7 +21,7 @@ OBJDIR = os.path.join(LIBDIR, "obj")
 LIB = os.path.join(LIBDIR, "libmsacl_b200.so")
 STAMP = LIB + ".stamp"
 SOURCES = ["env_step.cu", "rollout_fused.cu", "windows.cu", "targets.cu", "tc_selftest.cu", "rollout_tc.cu",
-           "mlp_tc.cu", "mlp_bwd.cu", "learner.cu", "certify.cu"]
+           "mlp_tc.cu", "mlp_bwd.cu", "learner.cu", "certify.cu", "certify_region.cu"]
 SOURCES = [s for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh")) + [os.path.join(ROOT, "include", "msacl_b200.h")]
 

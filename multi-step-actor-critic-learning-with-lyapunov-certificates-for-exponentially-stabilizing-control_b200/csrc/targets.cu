@@ -567,6 +567,32 @@ __global__ void __launch_bounds__(256) ffma2_probe_outer_kernel(int iters, const
   if (s == 123.456f) sink[0] = s;
 }
 
+// mode 8: the mode-1 outer product with directed rounding, half FFMA.RM (__fmaf_rd) and half FFMA.RP (__fmaf_ru): the issue
+// rate of the interval GEMMs of certify_region.cu
+__global__ void __launch_bounds__(256) ffma_rmrp_probe_outer_kernel(int iters, const float* __restrict__ src, float* sink) {
+  float a[8], b[8], acc[8][8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) { a[j] = src[(threadIdx.x + j) & 63]; b[j] = src[(threadIdx.x * 3 + j) & 63]; }
+#pragma unroll
+  for (int i = 0; i < 8; ++i)
+#pragma unroll
+    for (int c = 0; c < 8; ++c) acc[i][c] = 0.f;
+  for (int it = 0; it < iters; ++it) {
+#pragma unroll
+    for (int u = 0; u < 2; ++u)
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int c = 0; c < 8; ++c) acc[i][c] = (i & 1) ? __fmaf_ru(a[i], b[c], acc[i][c]) : __fmaf_rd(a[i], b[c], acc[i][c]);
+  }
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < 8; ++i)
+#pragma unroll
+    for (int c = 0; c < 8; ++c) s += acc[i][c];
+  if (s == 123.456f) sink[0] = s;
+}
+
 // mode 3: FP64 DFMA throughput (8 independent chains per thread)
 __global__ void __launch_bounds__(256) dfma_probe_kernel(int iters, float* sink) {
   double a[8];
@@ -733,7 +759,13 @@ extern "C" int msacl_polyak_update(int32_t count, const float* const* src, float
 }
 
 extern "C" int msacl_ffma_probe(int32_t mode, int32_t iters, float* sink, double* flops, void* stream) {
-  if (iters <= 0 || !sink || mode < 0 || mode > 7) { set_error("ffma_probe: bad argument"); return MSACL_ERR_BAD_ARG; }
+  if (iters <= 0 || !sink || mode < 0 || mode > 8) { set_error("ffma_probe: bad argument"); return MSACL_ERR_BAD_ARG; }
+  if (mode == 8) {
+    const unsigned grid = 2 * kNumSMs * 4;
+    ffma_rmrp_probe_outer_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(iters, sink + 64, sink);
+    if (flops) *flops = 2.0 * 128.0 * (double)iters * 256.0 * (double)grid;
+    return check_launch("ffma_probe");
+  }
   if (mode >= 4) {          // one warp per sub-partition: 148 blocks x 128 threads; *flops = FP64 instructions per warp
     if (mode == 4) dmul_dadd_probe_kernel<8><<<kNumSMs, 128, 0, (cudaStream_t)stream>>>(iters, sink);
     else if (mode == 5) dmul_dadd_probe_kernel<2><<<kNumSMs, 128, 0, (cudaStream_t)stream>>>(iters, sink);

@@ -6,6 +6,11 @@
 The checkpoint is the trainer's `apprfunc_{iteration}.pkl` (`networks.state_dict()`); it is loaded into an ApproxContainer
 built with the network arguments of examples/msacl_train_b200.py (reference defaults, lyapunov_output_dim 256; override
 with the flags below).  The result is an empirical check over the sampled initial states and the horizon, not a proof.
+
+With --region LO HI the sound region verifier runs instead (interval branch-and-bound over the box [LO, HI]^obs_dim minus
+the inner box --inner, for --steps closed-loop steps, cells down to --max_depth) and its RegionReport is printed:
+
+    python tools/certify.py --env_name VanderPol --checkpoint apprfunc_2000.pkl --region -2 2 --inner 0.1 --max_depth 30
 """
 import argparse
 import json
@@ -44,9 +49,23 @@ def main(argv=None):
                    "(box envs) instead of the env's reset distribution")
     p.add_argument("--lyapunov_output_dim", type=int, default=256)
     p.add_argument("--rollout_engine", default="tc")
+    p.add_argument("--region", type=float, nargs=2, metavar=("LO", "HI"), help="run the sound region verifier over "
+                   "[LO, HI]^obs_dim instead of the sampling check")
+    p.add_argument("--inner", type=float, nargs="+", metavar="R", help="inner box B: a radius R, or LO HI (default 0.05 of "
+                   "the box width)")
+    p.add_argument("--steps", type=int, default=1, help="closed-loop steps m of the region verifier")
+    p.add_argument("--max_depth", type=int, default=30, help="deepest cell of the region verifier")
     a = p.parse_args(argv)
     nets = ApproxContainer(**network_kwargs(a.env_name, a.lyapunov_output_dim)).cuda()
     nets.load_state_dict(torch.load(a.checkpoint, map_location="cuda", weights_only=True))
+    if a.region:
+        kw = dict(networks=nets, env_name=a.env_name, box=tuple(a.region), lya_eta=a.lya_eta, alpha1=a.alpha1, alpha2=a.alpha2,
+                  steps=a.steps, max_depth=a.max_depth)
+        if a.inner:
+            kw["inner"] = a.inner[0] if len(a.inner) == 1 else tuple(a.inner[:2])
+        rep = msacl_b200.create_region_certifier(**kw).run()
+        print(rep.to_json(), flush=True)
+        return json.loads(rep.to_json())
     ver = msacl_b200.create_certifier(networks=nets, env_name=a.env_name, num_states=a.num_states, horizon=a.horizon,
                                       lya_eta=a.lya_eta, alpha1=a.alpha1, alpha2=a.alpha2, v_atol=a.v_atol, seed=a.seed,
                                       init=("box", a.box[0], a.box[1]) if a.box else "reset", rollout_engine=a.rollout_engine)
