@@ -480,6 +480,15 @@ int msacl_certify_roa(int64_t n, const float* v0, float c_star, int64_t* summary
  * their stored float32 parameters, exact sin / cos / tanh, the Euler map in exact arithmetic (the env's constants read as
  * exact reals).  The rounding of any float implementation (split-bf16 rollout GEMMs, float32 env kernels) is not modelled.
  * Envs: VanderPol, Pendulum, DuctedFan, TwoLink.
+ *
+ * Bounded disturbances (the *_robust entry points, msacl_region_disturbance_t): one disturbed closed-loop step is
+ *   F_d(x) = Phi(x, clip(half tanh(mu(x + n)) + mid) + u) + w,   n in N, u in U, w in W
+ * with Phi the CONTROL_STEP Euler map.  n is sensor noise seen by the policy only (V is evaluated at the true state); u is an
+ * actuator disturbance added after the clip, not re-clipped, and held over the sub-steps; w is a process disturbance added
+ * once after the sub-steps.  N, U, W are boxes (need not contain 0), and each of the m steps takes its own (n, u, w): every
+ * condition above, LEAVES, the inner-cell conditions and c_in hold for EVERY admissible disturbance sequence.  A REFUTE flag
+ * still evaluates the degenerate [c, c] with the sets as intervals, so its violation holds for every sequence and its margin
+ * is the least violation over them.  With all three sets {0} the results equal those of the plain entry points bit for bit.
  * --------------------------------------------------------------------------------------------------------------- */
 enum {
   MSACL_REGION_NONFINITE = 1,         /* cell flags (msacl_region_out_t.flags) */
@@ -554,6 +563,12 @@ typedef struct {                      /* scratch of one msacl_region_round for k
   int64_t* scan;                      /* [3 * (k / 256 + 1) + 8] */
 } msacl_region_ws_t;
 
+typedef struct {                      /* disturbance boxes [lo, hi] of the *_robust entry points (finite, lo <= hi) */
+  float obs_lo[16], obs_hi[16];       /* N, [obs_dim]: sensor noise added to the policy's input */
+  float act_lo[2], act_hi[2];         /* U, [act_dim]: actuator disturbance added to the clipped action */
+  float state_lo[16], state_hi[16];   /* W, [obs_dim]: process disturbance added to the state after the Euler sub-steps */
+} msacl_region_disturbance_t;
+
 /* Bytes of the packed network image (floats, 16-byte aligned). */
 int64_t msacl_region_image_bytes(void);
 /* Pack the policy and V net into the image: zero-padded to 256 units, the 256-wide matrices as [k][W+ | W-] rows. */
@@ -569,6 +584,13 @@ int msacl_region_eval(const msacl_region_params_t* p, const float* image, int64_
 int msacl_region_round(const msacl_region_params_t* p, const msacl_region_bnb_t* b, const float* image, uint32_t* stack,
                        int64_t top, int64_t k, const msacl_region_ws_t* ws, int64_t* stats, float* examples, int64_t* children,
                        void* stream);
+/* msacl_region_eval and msacl_region_round under the bounded disturbances *w (see above; the trace's a is the disturbed
+ * action, its F^j the disturbed state).  MSACL_ERR_BAD_ARG for a non-finite bound or lo > hi. */
+int msacl_region_eval_robust(const msacl_region_params_t* p, const float* image, int64_t n, const int64_t* n_dev, const float* lo,
+                             const float* hi, const msacl_region_out_t* out, void* stream, const msacl_region_disturbance_t* w);
+int msacl_region_round_robust(const msacl_region_params_t* p, const msacl_region_bnb_t* b, const float* image, uint32_t* stack,
+                              int64_t top, int64_t k, const msacl_region_ws_t* ws, int64_t* stats, float* examples,
+                              int64_t* children, void* stream, const msacl_region_disturbance_t* w);
 
 const char* msacl_last_error(void);
 int msacl_abi_version(void);

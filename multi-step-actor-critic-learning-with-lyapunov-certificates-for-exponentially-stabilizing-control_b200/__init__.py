@@ -78,6 +78,9 @@ def create_region_certifier(**kwargs):
     """Sound region verifier of the Lyapunov certificate (no counterpart in the reference): interval branch-and-bound over
     the cells of a state box X0 \\ B, proving V's (1 - eta)^m decrease over m greedy closed-loop steps for every state of a
     verified cell, for the real-arithmetic closed loop.  `create_region_certifier(networks=..., env_name=..., box=(lo, hi),
-    inner=r).run()` -> RegionReport."""
+    inner=r).run()` -> RegionReport.  With `disturbance=dict(obs=..., act=..., state=...)` (sensor noise, actuator and
+    process disturbance boxes: a radius r for [-r, r] or a (lo, hi) tuple) every statement holds for every admissible
+    disturbance sequence and run() returns a RobustRegionReport; `.robustness_margin(s_max)` bisects the largest proven scale
+    of those boxes."""
     from .certify_region import B200RegionVerifier
     return B200RegionVerifier(**kwargs)

@@ -86,6 +86,11 @@ class RegionWs(C.Structure):
                 ("probe", vp), ("status", vp), ("scan", vp)]
 
 
+class RegionDisturbance(C.Structure):
+    _fields_ = [("obs_lo", C.c_float * 16), ("obs_hi", C.c_float * 16), ("act_lo", C.c_float * 2), ("act_hi", C.c_float * 2),
+                ("state_lo", C.c_float * 16), ("state_hi", C.c_float * 16)]
+
+
 f32 = C.c_float
 i32, i64 = C.c_int32, C.c_int64
 
@@ -155,6 +160,10 @@ SIGNATURES = {
     "msacl_region_eval": (C.c_int, [C.POINTER(RegionParams), vp, i64, vp, vp, vp, C.POINTER(RegionOut), vp]),
     "msacl_region_round": (C.c_int, [C.POINTER(RegionParams), C.POINTER(RegionBnb), vp, vp, i64, i64, C.POINTER(RegionWs), vp, vp,
                                      vp, vp]),
+    "msacl_region_eval_robust": (C.c_int, [C.POINTER(RegionParams), vp, i64, vp, vp, vp, C.POINTER(RegionOut), vp,
+                                           C.POINTER(RegionDisturbance)]),
+    "msacl_region_round_robust": (C.c_int, [C.POINTER(RegionParams), C.POINTER(RegionBnb), vp, vp, i64, i64, C.POINTER(RegionWs), vp,
+                                            vp, vp, vp, C.POINTER(RegionDisturbance)]),
 }
 
 

@@ -34,6 +34,19 @@ c_sound, then S = {x in X0 : V(x) < c_sound} is forward invariant under F^m, and
 
 The frontier is a stack of at most max_cells cells, processed depth-first in chunks.  The actor and V net are packed from
 the CURRENT parameters on every `run()`.
+
+BOUNDED DISTURBANCES (`disturbance=dict(obs=..., act=..., state=...)`).  One disturbed closed-loop step is
+
+  F_d(x) = Phi(x, clip(half tanh(mu(x + n)) + mid) + u) + w,   n in N, u in U, w in W
+
+with Phi the CONTROL_STEP Euler map: n is sensor noise that only the policy sees (V is evaluated at the true state), u an
+actuator disturbance added after the clip (not re-clipped, held over the sub-steps), w a process disturbance added once after
+the sub-steps.  N, U, W are boxes, possibly asymmetric and not containing 0 (a constant bias), and each of the m steps takes
+its own (n, u, w).  Every condition -- DECREASE, ESCAPED, LEAVES, the inner-cell conditions, c_in -- then holds for EVERY
+admissible disturbance sequence, and the invariance statement becomes robust invariance of S plus the ultimate bound
+{V <= reach_level} (practical stability).  A counterexample is still the centre [c, c] with the sets as intervals: its
+violation holds for every sequence, and its margin is the least violation over them.  With all sets {0} the verifier is the
+nominal one, bit for bit.
 """
 import ctypes as C
 import json
@@ -151,6 +164,68 @@ class RegionReport:
                    reach_level=max(c_in, v_inner) if invariant else None, counterexamples=examples)
 
 
+@dataclass
+class RobustRegionReport(RegionReport):
+    """RegionReport of a run under bounded disturbances: every statement holds for every admissible disturbance sequence."""
+    disturbance: dict = field(default_factory=dict)     # {"obs" | "act" | "state": [lo list, hi list]}: the proven boxes
+
+
+@dataclass
+class RobustnessMargin:
+    """Result of B200RegionVerifier.robustness_margin (every scale is that of a full run)."""
+    s_proven: object              # largest tested scale whose run proved invariance with c_sound >= level; None if s = 0 failed
+    s_failed: object              # smallest tested scale whose run did not; None if s_max passed
+    runs: int
+    report: RobustRegionReport    # the run at s_proven (at s = 0 when the nominal loop is not proven)
+    nominal_proven: bool
+
+
+DIST_KEYS = ("obs", "act", "state")
+
+
+def _f32_out(x, down):
+    """float32 array of x rounded outward (down for lower bounds), so the proven box contains the requested one."""
+    x = np.asarray(x, np.float64)
+    f = x.astype(np.float32)
+    bad = f.astype(np.float64) > x if down else f.astype(np.float64) < x
+    return np.where(bad, np.nextafter(f, np.float32(-np.inf if down else np.inf)), f).astype(np.float32)
+
+
+def parse_disturbance(dist, obs_dim, act_dim):
+    """{"obs" | "act" | "state": (lo, hi) float32 arrays} from the user's dict: each entry is a radius r >= 0 (scalar, or a list
+    / array per dimension) meaning [-r, r], or a tuple (lo, hi) of scalars or per-dimension values; missing keys are {0}.
+    Bounds are rounded outward to float32."""
+    if not isinstance(dist, dict):
+        raise ValueError(f"disturbance must be a dict with keys {DIST_KEYS}, got {type(dist).__name__}")
+    unknown = set(dist) - set(DIST_KEYS)
+    if unknown:
+        raise ValueError(f"disturbance: unknown keys {sorted(unknown)}; allowed: {DIST_KEYS}")
+    out = {}
+    for key, n in zip(DIST_KEYS, (obs_dim, act_dim, obs_dim)):
+        v = dist.get(key, 0.0)
+        if isinstance(v, tuple):
+            if len(v) != 2:
+                raise ValueError(f"disturbance {key}: a (lo, hi) pair needs 2 entries, got {len(v)}")
+            lo, hi = (np.asarray(b, np.float64) for b in v)
+        else:
+            r = np.asarray(v, np.float64)
+            if np.any(r < 0):
+                raise ValueError(f"disturbance {key}: a radius must be >= 0, got {r.tolist()}")
+            lo, hi = -r, r
+        vals = []
+        for b in (lo, hi):
+            if b.ndim > 1 or (b.ndim == 1 and b.shape[0] not in (1, n)):
+                raise ValueError(f"disturbance {key}: need a scalar or {n} values per bound, got shape {list(b.shape)}")
+            vals.append(np.broadcast_to(b, (n,)).astype(np.float64))
+        lo, hi = vals
+        if not (np.all(np.isfinite(lo)) and np.all(np.isfinite(hi))):
+            raise ValueError(f"disturbance {key}: bounds must be finite, got [{lo.tolist()}, {hi.tolist()}]")
+        if not np.all(lo <= hi):
+            raise ValueError(f"disturbance {key}: need lo <= hi, got [{lo.tolist()}, {hi.tolist()}]")
+        out[key] = (_f32_out(lo, True), _f32_out(hi, False))
+    return out
+
+
 def _layers(seq, what):
     lin = [m for m in seq if isinstance(m, torch.nn.Linear)]
     other = [m for m in seq if not isinstance(m, torch.nn.Linear)]
@@ -170,7 +245,9 @@ class B200RegionVerifier:
     [-r, r]^D; default 0.05 of the box width around the origin), lya_eta (0.15, in (0, 1)), alpha1 (1), alpha2 (2), steps
     (m, 1), max_depth (30, <= 50), max_cells (2^22: frontier capacity), max_examples (16), chunk (cells per round, default
     max_cells // (2 (max_depth + 1))), device ("cuda"), trace (optional callable(lo, hi, status) with device views of every
-    round's cell boxes and their status, for tests and inspection)."""
+    round's cell boxes and their status, for tests and inspection), disturbance (optional dict with keys obs / act / state:
+    the boxes N, U, W of the module docstring, each a radius r >= 0 -- scalar, or a list / array per dimension -- for
+    [-r, r], or a tuple (lo, hi); missing keys are {0}; run() then returns a RobustRegionReport)."""
 
     def __init__(self, **kw):
         self.networks = kw["networks"]
@@ -236,6 +313,8 @@ class B200RegionVerifier:
         if self.v_lin[0].in_features != D:
             raise ValueError(f"lyapunov: input width {self.v_lin[0].in_features} != obs_dim {D}")
         self.v_tanh = isinstance(vact, torch.nn.Tanh)
+        dist = kw.get("disturbance")
+        self.disturbance = None if dist is None else parse_disturbance(dist, D, spec.act_dim)
         self._lib = None
 
     # ---- device plumbing
@@ -246,6 +325,18 @@ class B200RegionVerifier:
         for d in range(self.spec.obs_dim):
             p.x0_lo[d], p.x0_hi[d] = float(self.box[0][d]), float(self.box[1][d])
         return p
+
+    def _dist(self, dist):
+        d = _lib.RegionDisturbance()
+        for key, (lo, hi) in dist.items():
+            for j in range(lo.shape[0]):
+                getattr(d, key + "_lo")[j], getattr(d, key + "_hi")[j] = float(lo[j]), float(hi[j])
+        return d
+
+    def _scaled(self, s):
+        """The disturbance boxes times s >= 0, rounded outward to float32."""
+        return {k: (_f32_out(np.float64(s) * lo.astype(np.float64), True), _f32_out(np.float64(s) * hi.astype(np.float64), False))
+                for k, (lo, hi) in self.disturbance.items()}
 
     def pack(self):
         """The network image from the current parameters (device float tensor)."""
@@ -278,14 +369,59 @@ class B200RegionVerifier:
         """Enclosures for the boxes [lo, hi] ([n, D] float32 CUDA): dict of device tensors (v_lo, v_hi, vm_lo, vm_hi, img_lo,
         img_hi, flags, margin and, with trace, [n, m, 4A + 2D] = mu lo, mu hi, a lo, a hi, F^j lo, F^j hi)."""
         image = self.pack() if image is None else image
+        self._lib = self._lib or _lib.load()
         lo, hi = lo.float().contiguous(), hi.float().contiguous()
         o, desc = self._out(lo.shape[0], trace)
         p = self.params()
-        _lib.check(self._lib.msacl_region_eval(C.byref(p), image.data_ptr(), lo.shape[0], None, lo.data_ptr(), hi.data_ptr(),
-                                               C.byref(desc), _lib.current_stream()))
+        args = (C.byref(p), image.data_ptr(), lo.shape[0], None, lo.data_ptr(), hi.data_ptr(), C.byref(desc), _lib.current_stream())
+        if self.disturbance is None:
+            _lib.check(self._lib.msacl_region_eval(*args))
+        else:
+            _lib.check(self._lib.msacl_region_eval_robust(*args, C.byref(self._dist(self.disturbance))))
         return o
 
     def run(self) -> RegionReport:
+        """Verify the region: a RegionReport, or a RobustRegionReport when the verifier has a disturbance."""
+        return self._run(self.disturbance)
+
+    def run_scaled(self, s) -> RobustRegionReport:
+        """run() with every disturbance box scaled by s >= 0 (s = 0 is the nominal loop)."""
+        if self.disturbance is None:
+            raise ValueError("run_scaled needs a verifier created with a disturbance")
+        return self._run(self._scaled(s))
+
+    def robustness_margin(self, s_max, iters=8, level=0.0) -> RobustnessMargin:
+        """Bisect the scale s in [0, s_max] of the disturbance shape for the largest s whose run proves `invariant` with
+        c_sound >= level.  Runs s = 0 (the nominal loop) first: if that is not proven there is no margin (s_proven None).
+        Then s_max, then `iters` bisection steps.  Every reported scale is that of a full run, and each such run is a sound
+        statement at its own scale; whether the proof is monotone in s (a larger set can only lose) only decides how tight
+        the bracket [s_proven, s_failed] is, not whether s_proven is sound."""
+        s_max = float(s_max)
+        if not (s_max > 0 and math.isfinite(s_max)):
+            raise ValueError("s_max must be positive and finite")
+        if int(iters) < 0:
+            raise ValueError("iters must be >= 0")
+        ok = lambda r: bool(r.invariant) and r.c_sound != "none" and r.c_sound >= level
+        runs = 1
+        rep = self.run_scaled(0.0)
+        if not ok(rep):
+            return RobustnessMargin(s_proven=None, s_failed=0.0, runs=runs, report=rep, nominal_proven=False)
+        good, good_rep, bad = 0.0, rep, s_max
+        rep = self.run_scaled(s_max)
+        runs += 1
+        if ok(rep):
+            return RobustnessMargin(s_proven=s_max, s_failed=None, runs=runs, report=rep, nominal_proven=True)
+        for _ in range(int(iters)):
+            mid = 0.5 * (good + bad)
+            rep = self.run_scaled(mid)
+            runs += 1
+            if ok(rep):
+                good, good_rep = mid, rep
+            else:
+                bad = mid
+        return RobustnessMargin(s_proven=good, s_failed=bad, runs=runs, report=good_rep, nominal_proven=True)
+
+    def _run(self, dist):
         D, dev = self.spec.obs_dim, self.device
         W = 1 + D
         image = self.pack()
@@ -311,13 +447,17 @@ class B200RegionVerifier:
                    scan=torch.zeros(3 * nb + 8, dtype=torch.int64, device=dev))
         ws = _lib.RegionWs(res=rdesc, pres=pdesc, **{k: v.data_ptr() for k, v in wsb.items()})
         top, rounds = 1, 0
+        wd = None if dist is None else self._dist(dist)
         while top > 0:
             k = min(K, top, self.max_cells - top)
             if k < 1:
                 raise RuntimeError(f"region verifier: the frontier exceeds max_cells = {self.max_cells}")
-            _lib.check(self._lib.msacl_region_round(C.byref(p), C.byref(b), image.data_ptr(), stack.data_ptr(), top, k, C.byref(ws),
-                                                    stats.data_ptr(), examples.data_ptr(), children.data_ptr(),
-                                                    _lib.current_stream()))
+            args = (C.byref(p), C.byref(b), image.data_ptr(), stack.data_ptr(), top, k, C.byref(ws), stats.data_ptr(),
+                    examples.data_ptr(), children.data_ptr(), _lib.current_stream())
+            if wd is None:
+                _lib.check(self._lib.msacl_region_round(*args))
+            else:
+                _lib.check(self._lib.msacl_region_round_robust(*args, C.byref(wd)))
             if self.trace is not None:
                 self.trace(wsb["lo"][:k], wsb["hi"][:k], wsb["status"][:k])
             rounds += 1
@@ -325,8 +465,12 @@ class B200RegionVerifier:
         s = stats.cpu().tolist()
         ex = examples[:min(self.max_examples, s[ST["refuted"]])].cpu().numpy()
         exs = [{"x": r[:D].tolist(), "kind": "decrease" if r[D + 1] == 1.0 else "escaped", "margin": float(r[D])} for r in ex]
-        rep = RegionReport.from_stats(s, exs, env_name=self.env_name, box=[self.box[0].tolist(), self.box[1].tolist()],
-                                      inner=[blo, bhi], steps=self.steps, lya_eta=self.lya_eta, alpha1=self.alpha1,
-                                      alpha2=self.alpha2, max_depth=self.max_depth)
+        meta = dict(env_name=self.env_name, box=[self.box[0].tolist(), self.box[1].tolist()], inner=[blo, bhi], steps=self.steps,
+                    lya_eta=self.lya_eta, alpha1=self.alpha1, alpha2=self.alpha2, max_depth=self.max_depth)
+        if dist is None:
+            rep = RegionReport.from_stats(s, exs, **meta)
+        else:
+            rep = RobustRegionReport.from_stats(s, exs, **meta,
+                                                disturbance={k: [lo.tolist(), hi.tolist()] for k, (lo, hi) in dist.items()})
         rep.rounds, rep.evaluated = rounds, s[ST["evaluated"]]
         return rep

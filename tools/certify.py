@@ -11,6 +11,13 @@ With --region LO HI the sound region verifier runs instead (interval branch-and-
 the inner box --inner, for --steps closed-loop steps, cells down to --max_depth) and its RegionReport is printed:
 
     python tools/certify.py --env_name VanderPol --checkpoint apprfunc_2000.pkl --region -2 2 --inner 0.1 --max_depth 30
+
+--dist_obs, --dist_act and --dist_state (half-widths: one value, or one per dimension) run it under bounded sensor noise,
+actuator and process disturbances; the line then has a "disturbance" field.  --margin S_MAX bisects the largest scale
+s in [0, S_MAX] of those boxes that is still proven invariant and adds a "margin" field (s_proven is null with
+"nominal_proven": false when the undisturbed loop is not proven); the report is that of the run at s_proven:
+
+    python tools/certify.py --env_name VanderPol --checkpoint apprfunc_2000.pkl --region -1 1 --dist_state 1e-3 --margin 0.1
 """
 import argparse
 import json
@@ -55,6 +62,10 @@ def main(argv=None):
                    "the box width)")
     p.add_argument("--steps", type=int, default=1, help="closed-loop steps m of the region verifier")
     p.add_argument("--max_depth", type=int, default=30, help="deepest cell of the region verifier")
+    for key, what in (("obs", "sensor noise"), ("act", "actuator disturbance"), ("state", "process disturbance")):
+        p.add_argument(f"--dist_{key}", type=float, nargs="+", metavar="R", help=f"region verifier: {what} half-widths")
+    p.add_argument("--margin", type=float, metavar="S_MAX", help="region verifier: bisect the proven scale of the "
+                   "disturbance in [0, S_MAX]")
     a = p.parse_args(argv)
     nets = ApproxContainer(**network_kwargs(a.env_name, a.lyapunov_output_dim)).cuda()
     nets.load_state_dict(torch.load(a.checkpoint, map_location="cuda", weights_only=True))
@@ -63,9 +74,21 @@ def main(argv=None):
                   steps=a.steps, max_depth=a.max_depth)
         if a.inner:
             kw["inner"] = a.inner[0] if len(a.inner) == 1 else tuple(a.inner[:2])
-        rep = msacl_b200.create_region_certifier(**kw).run()
-        print(rep.to_json(), flush=True)
-        return json.loads(rep.to_json())
+        dist = {k: getattr(a, f"dist_{k}") for k in ("obs", "act", "state") if getattr(a, f"dist_{k}") is not None}
+        if dist:
+            kw["disturbance"] = dist
+        elif a.margin is not None:
+            p.error("--margin needs --dist_obs, --dist_act or --dist_state")
+        ver = msacl_b200.create_region_certifier(**kw)
+        if a.margin is None:
+            rep = ver.run()
+            print(rep.to_json(), flush=True)
+            return json.loads(rep.to_json())
+        r = ver.robustness_margin(a.margin)
+        out = json.loads(r.report.to_json())
+        out["margin"] = dict(s_max=a.margin, s_proven=r.s_proven, s_failed=r.s_failed, runs=r.runs, nominal_proven=r.nominal_proven)
+        print(json.dumps(out), flush=True)
+        return out
     ver = msacl_b200.create_certifier(networks=nets, env_name=a.env_name, num_states=a.num_states, horizon=a.horizon,
                                       lya_eta=a.lya_eta, alpha1=a.alpha1, alpha2=a.alpha2, v_atol=a.v_atol, seed=a.seed,
                                       init=("box", a.box[0], a.box[1]) if a.box else "reset", rollout_engine=a.rollout_engine)
