@@ -9,7 +9,7 @@ import os
 from . import build as _build
 
 _LIB = None
-ABI_VERSION = 2      # MSACL_ABI_VERSION of include/msacl_b200.h this binding was written against
+ABI_VERSION = 3      # MSACL_ABI_VERSION of include/msacl_b200.h this binding was written against
 
 c_f32p = C.POINTER(C.c_float)
 c_f64p = C.POINTER(C.c_double)
@@ -65,10 +65,15 @@ class RegionNets(C.Structure):
                 ("v_w1", vp), ("v_b1", vp), ("v_w2", vp), ("v_b2", vp), ("v_w3", vp), ("v_b3", vp)]
 
 
+class RegionDisturbance(C.Structure):
+    _fields_ = [("obs_lo", C.c_float * 16), ("obs_hi", C.c_float * 16), ("act_lo", C.c_float * 2), ("act_hi", C.c_float * 2),
+                ("state_lo", C.c_float * 16), ("state_hi", C.c_float * 16)]
+
+
 class RegionParams(C.Structure):
     _fields_ = [("env_id", C.c_int32), ("steps", C.c_int32), ("v_tanh", C.c_int32), ("decay_lo", C.c_double),
                 ("decay_hi", C.c_double), ("alpha1", C.c_double), ("alpha2", C.c_double), ("x0_lo", C.c_float * 16),
-                ("x0_hi", C.c_float * 16)]
+                ("x0_hi", C.c_float * 16), ("dist", RegionDisturbance)]
 
 
 class RegionOut(C.Structure):
@@ -84,11 +89,6 @@ class RegionBnb(C.Structure):
 class RegionWs(C.Structure):
     _fields_ = [("cells", vp), ("lo", vp), ("hi", vp), ("res", RegionOut), ("plo", vp), ("phi", vp), ("pres", RegionOut),
                 ("probe", vp), ("status", vp), ("scan", vp)]
-
-
-class RegionDisturbance(C.Structure):
-    _fields_ = [("obs_lo", C.c_float * 16), ("obs_hi", C.c_float * 16), ("act_lo", C.c_float * 2), ("act_hi", C.c_float * 2),
-                ("state_lo", C.c_float * 16), ("state_hi", C.c_float * 16)]
 
 
 f32 = C.c_float
@@ -160,10 +160,6 @@ SIGNATURES = {
     "msacl_region_eval": (C.c_int, [C.POINTER(RegionParams), vp, i64, vp, vp, vp, C.POINTER(RegionOut), vp]),
     "msacl_region_round": (C.c_int, [C.POINTER(RegionParams), C.POINTER(RegionBnb), vp, vp, i64, i64, C.POINTER(RegionWs), vp, vp,
                                      vp, vp]),
-    "msacl_region_eval_robust": (C.c_int, [C.POINTER(RegionParams), vp, i64, vp, vp, vp, C.POINTER(RegionOut), vp,
-                                           C.POINTER(RegionDisturbance)]),
-    "msacl_region_round_robust": (C.c_int, [C.POINTER(RegionParams), C.POINTER(RegionBnb), vp, vp, i64, i64, C.POINTER(RegionWs), vp,
-                                            vp, vp, vp, C.POINTER(RegionDisturbance)]),
 }
 
 

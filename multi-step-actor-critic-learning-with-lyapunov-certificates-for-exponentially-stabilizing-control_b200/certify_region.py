@@ -318,20 +318,17 @@ class B200RegionVerifier:
         self._lib = None
 
     # ---- device plumbing
-    def params(self):
+    def params(self, dist=None):
+        """The kernel parameters, with the disturbance boxes `dist` ({"obs" | "act" | "state": (lo, hi)}; None leaves them 0)."""
         lo, hi = decay_bounds(self.lya_eta, self.steps)
         p = _lib.RegionParams(env_id=self.spec.env_id, steps=self.steps, v_tanh=int(self.v_tanh), decay_lo=lo, decay_hi=hi,
                               alpha1=self.alpha1, alpha2=self.alpha2)
         for d in range(self.spec.obs_dim):
             p.x0_lo[d], p.x0_hi[d] = float(self.box[0][d]), float(self.box[1][d])
+        for key, (dlo, dhi) in (dist or {}).items():
+            for j in range(dlo.shape[0]):
+                getattr(p.dist, key + "_lo")[j], getattr(p.dist, key + "_hi")[j] = float(dlo[j]), float(dhi[j])
         return p
-
-    def _dist(self, dist):
-        d = _lib.RegionDisturbance()
-        for key, (lo, hi) in dist.items():
-            for j in range(lo.shape[0]):
-                getattr(d, key + "_lo")[j], getattr(d, key + "_hi")[j] = float(lo[j]), float(hi[j])
-        return d
 
     def _scaled(self, s):
         """The disturbance boxes times s >= 0, rounded outward to float32."""
@@ -372,12 +369,9 @@ class B200RegionVerifier:
         self._lib = self._lib or _lib.load()
         lo, hi = lo.float().contiguous(), hi.float().contiguous()
         o, desc = self._out(lo.shape[0], trace)
-        p = self.params()
-        args = (C.byref(p), image.data_ptr(), lo.shape[0], None, lo.data_ptr(), hi.data_ptr(), C.byref(desc), _lib.current_stream())
-        if self.disturbance is None:
-            _lib.check(self._lib.msacl_region_eval(*args))
-        else:
-            _lib.check(self._lib.msacl_region_eval_robust(*args, C.byref(self._dist(self.disturbance))))
+        p = self.params(self.disturbance)
+        _lib.check(self._lib.msacl_region_eval(C.byref(p), image.data_ptr(), lo.shape[0], None, lo.data_ptr(), hi.data_ptr(),
+                                               C.byref(desc), _lib.current_stream()))
         return o
 
     def run(self) -> RegionReport:
@@ -425,7 +419,7 @@ class B200RegionVerifier:
         D, dev = self.spec.obs_dim, self.device
         W = 1 + D
         image = self.pack()
-        p = self.params()
+        p = self.params(dist)
         glo, ghi, blo, bhi = self.inner_grid
         b = _lib.RegionBnb(max_depth=self.max_depth, inner_level=self.inner_level, max_examples=self.max_examples)
         for d in range(D):
@@ -447,17 +441,13 @@ class B200RegionVerifier:
                    scan=torch.zeros(3 * nb + 8, dtype=torch.int64, device=dev))
         ws = _lib.RegionWs(res=rdesc, pres=pdesc, **{k: v.data_ptr() for k, v in wsb.items()})
         top, rounds = 1, 0
-        wd = None if dist is None else self._dist(dist)
         while top > 0:
             k = min(K, top, self.max_cells - top)
             if k < 1:
                 raise RuntimeError(f"region verifier: the frontier exceeds max_cells = {self.max_cells}")
-            args = (C.byref(p), C.byref(b), image.data_ptr(), stack.data_ptr(), top, k, C.byref(ws), stats.data_ptr(),
-                    examples.data_ptr(), children.data_ptr(), _lib.current_stream())
-            if wd is None:
-                _lib.check(self._lib.msacl_region_round(*args))
-            else:
-                _lib.check(self._lib.msacl_region_round_robust(*args, C.byref(wd)))
+            _lib.check(self._lib.msacl_region_round(C.byref(p), C.byref(b), image.data_ptr(), stack.data_ptr(), top, k, C.byref(ws),
+                                                    stats.data_ptr(), examples.data_ptr(), children.data_ptr(),
+                                                    _lib.current_stream()))
             if self.trace is not None:
                 self.trace(wsb["lo"][:k], wsb["hi"][:k], wsb["status"][:k])
             rounds += 1

@@ -11,11 +11,10 @@
 // step (IEnv<ID>, one lane per cell) run on the same warps.  Tensor cores are not used: the rounding of tcgen05 FP32
 // accumulation is not specified, so no outward bound exists for it.
 //
-// Bounded disturbances (msacl_region_eval_robust / msacl_region_round_robust) widen one closed-loop step by three boxes:
-// N (sensor noise) the policy's layer-1 input, which the owner lanes write to sm.pl / sm.pu from the state box, so V and the
-// env step keep reading the un-widened state; U the clipped action; W the state after IEnv<ID>::step.  A set that is exactly
-// {0} is skipped by a uniform flag rather than added as [0, 0] (-0 + 0 rounded up is +0), so the nominal results are
-// bit-identical to those of the plain entry points, which run the same kernel with every flag off.
+// The bounded disturbances of p.dist widen one closed-loop step by three boxes: N (sensor noise) the policy's layer-1 input,
+// which the owner lanes write to sm.pl / sm.pu from the state box, so V and the env step keep reading the un-widened state;
+// U the clipped action; W the state after IEnv<ID>::step.  A set that is exactly {0} is skipped by a uniform flag rather than
+// added as [0, 0] (-0 + 0 rounded up is +0), so an all-zero p.dist runs the nominal closed loop bit for bit.
 //
 // The branch-and-bound round (msacl_region_round) is count / scan / scatter in the style of windows.cu: cells are dyadic
 // ([depth, idx per dimension], depth t bisects dimension t mod D -- the widest one scaled by the box width, lowest index on
@@ -63,10 +62,15 @@ struct RSmem {
   unsigned long long full_bar[RSTAGE], empty_bar[RSTAGE];
 };
 
-// the disturbance boxes and, per set, whether it is not exactly {0} (set on the host, uniform in the kernel)
+// per disturbance set of p.dist, whether it is not exactly {0} (set on the host, uniform in the kernel)
 struct RDist {
-  msacl_region_disturbance_t w;
   int obs, act, state;
+};
+// region_eval_kernel's parameters as one by-value argument: the flags are then loaded where they are used, whereas a small
+// argument of their own is held in registers over the whole kernel (VanderPol: 168 instead of 155)
+struct REval {
+  msacl_region_params_t p;
+  RDist on;
 };
 
 // ----------------------------------------------------------------------------------------------------------------------
@@ -107,7 +111,7 @@ __global__ void region_pack_kernel(msacl_region_nets_t s, float* img) {
 // ----------------------------------------------------------------------------------------------------------------------
 template <int ID, int VT>
 __global__ void __launch_bounds__(RT, 1)
-region_eval_kernel(msacl_region_params_t p, RDist dist, const float* __restrict__ img, int64_t n_host, const int64_t* n_dev,
+region_eval_kernel(REval args, const float* __restrict__ img, int64_t n_host, const int64_t* n_dev,
                    const float* __restrict__ in_lo, const float* __restrict__ in_hi, msacl_region_out_t out) {
   using E = Env<ID>;
   constexpr int D = E::D, A = E::A;
@@ -116,6 +120,8 @@ region_eval_kernel(msacl_region_params_t p, RDist dist, const float* __restrict_
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, m0 = warp * RC;
   const int64_t n = n_dev ? *n_dev : n_host;
   const int64_t tiles = (n + RTM - 1) / RTM;
+  const msacl_region_params_t& p = args.p;
+  const RDist& on = args.on;
   const int m = p.steps;
   if (tid == 0) {
 #pragma unroll
@@ -276,17 +282,17 @@ region_eval_kernel(msacl_region_params_t p, RDist dist, const float* __restrict_
     uint32_t flags = 0;
     float esc_margin = 0.f;
     for (int j = 1; j <= m; ++j) {
-      if (dist.obs) {
+      if (on.obs) {
         if (lane < RC) {
 #pragma unroll
           for (int d = 0; d < D; ++d) {
-            sm.pl[m0 + lane][d] = __fadd_rd(sm.xl[m0 + lane][d], dist.w.obs_lo[d]);
-            sm.pu[m0 + lane][d] = __fadd_ru(sm.xu[m0 + lane][d], dist.w.obs_hi[d]);
+            sm.pl[m0 + lane][d] = __fadd_rd(sm.xl[m0 + lane][d], p.dist.obs_lo[d]);
+            sm.pu[m0 + lane][d] = __fadd_ru(sm.xu[m0 + lane][d], p.dist.obs_hi[d]);
           }
         }
         __syncwarp();
       }
-      layer1(P_W1, P_B1, dist.obs ? sm.pl : sm.xl, dist.obs ? sm.pu : sm.xu);
+      layer1(P_W1, P_B1, on.obs ? sm.pl : sm.xl, on.obs ? sm.pu : sm.xu);
       act_store(false);
       gemm(P_B2);
       // ReLU, then the mean rows of the output layer (sign-selected) on the register tile
@@ -324,14 +330,14 @@ region_eval_kernel(msacl_region_params_t p, RDist dist, const float* __restrict_
           const If t = itanh(mean[q]);
           act[q] = {fminf(fmaxf(__fmaf_rd(half, t.l, mid), E::act_low(q)), E::act_high(q)),
                     fminf(fmaxf(__fmaf_ru(half, t.u, mid), E::act_low(q)), E::act_high(q))};
-          if (dist.act) act[q] = iadd(act[q], If{dist.w.act_lo[q], dist.w.act_hi[q]});   // after the clip, not re-clipped
+          if (on.act) act[q] = iadd(act[q], If{p.dist.act_lo[q], p.dist.act_hi[q]});   // after the clip, not re-clipped
         }
 #pragma unroll
         for (int d = 0; d < D; ++d) x[d] = If{sm.xl[m0 + lane][d], sm.xu[m0 + lane][d]};
         IEnv<ID>::step(x, act);
 #pragma unroll
         for (int d = 0; d < D; ++d) {
-          if (dist.state) x[d] = iadd(x[d], If{dist.w.state_lo[d], dist.w.state_hi[d]});
+          if (on.state) x[d] = iadd(x[d], If{p.dist.state_lo[d], p.dist.state_hi[d]});
           if (!(x[d].l > E::obs_low(d) && x[d].u < E::obs_high(d))) flags |= MSACL_REGION_ESCAPED;
           const float out_by = fmaxf(__fsub_rd(x[d].l, E::obs_high(d)), __fsub_rd(E::obs_low(d), x[d].u));
           if (out_by > 0.f) { flags |= MSACL_REGION_REFUTE_ESCAPED; esc_margin = fmaxf(esc_margin, out_by); }
@@ -595,7 +601,7 @@ __global__ void __launch_bounds__(RB) region_scatter_kernel(msacl_region_bnb_t b
 }
 
 template <int ID>
-static int eval_launch(const msacl_region_params_t* p, const RDist& dist, const float* image, int64_t n, const int64_t* n_dev,
+static int eval_launch(const msacl_region_params_t* p, const RDist& on, const float* image, int64_t n, const int64_t* n_dev,
                        const float* lo, const float* hi, const msacl_region_out_t* out, cudaStream_t s) {
   if constexpr (!IEnv<ID>::supported) {
     set_error("region_eval: env id %d is not supported (VanderPol, Pendulum, DuctedFan, TwoLink)", ID);
@@ -607,14 +613,16 @@ static int eval_launch(const msacl_region_params_t* p, const RDist& dist, const 
     auto launch = [&](auto kern) -> int {
       cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) { set_error("region_eval: smem attr: %s", cudaGetErrorString(e)); return (int)MSACL_ERR_CUDA; }
-      kern<<<grid, RT, smem, s>>>(*p, dist, image, n, n_dev, lo, hi, *out);
+      kern<<<grid, RT, smem, s>>>(REval{*p, on}, image, n, n_dev, lo, hi, *out);
       return check_launch("region_eval");
     };
     return p->v_tanh ? launch(region_eval_kernel<ID, 1>) : launch(region_eval_kernel<ID, 0>);
   }
 }
 
-static int check_params(const msacl_region_params_t* p, int* D) {
+// Refuses bad parameters, and a disturbance bound in the first obs_dim / act_dim entries of p->dist that is non-finite or has
+// lo > hi; *D = obs_dim, *on flags each disturbance set that is not exactly {0}.
+static int check_params(const msacl_region_params_t* p, int* D, RDist* on) {
   if (!p || p->steps < 1 || !(p->decay_lo > 0.0) || !(p->decay_hi >= p->decay_lo) || !(p->alpha1 > 0.0) || !(p->alpha2 > 0.0)) {
     set_error("region: bad parameters (need steps >= 1, 0 < decay_lo <= decay_hi, alpha1, alpha2 > 0)");
     return MSACL_ERR_BAD_ARG;
@@ -626,20 +634,11 @@ static int check_params(const msacl_region_params_t* p, int* D) {
     set_error("region: env id %d is not supported (VanderPol, Pendulum, DuctedFan, TwoLink)", p->env_id);
     return MSACL_ERR_BAD_ENV;
   }
-  return MSACL_OK;
-}
-
-// The kernel's view of w (NULL: no disturbance): refuses a non-finite bound or lo > hi in the first obs_dim / act_dim
-// entries, zeroes the rest, and flags each set that is not exactly {0}.
-static int make_dist(int env_id, const msacl_region_disturbance_t* w, RDist* r) {
-  *r = RDist{};
-  if (!w) return MSACL_OK;
-  int32_t dims[6];
-  if (int rc = msacl_env_dims(env_id, dims)) return rc;
-  const struct { const char* name; const float *lo, *hi; float *rlo, *rhi; int n; int* on; } sets[3] = {
-      {"obs", w->obs_lo, w->obs_hi, r->w.obs_lo, r->w.obs_hi, dims[0], &r->obs},
-      {"act", w->act_lo, w->act_hi, r->w.act_lo, r->w.act_hi, dims[1], &r->act},
-      {"state", w->state_lo, w->state_hi, r->w.state_lo, r->w.state_hi, dims[0], &r->state}};
+  const msacl_region_disturbance_t& w = p->dist;
+  *on = RDist{};
+  const struct { const char* name; const float *lo, *hi; int n; int* on; } sets[3] = {
+      {"obs", w.obs_lo, w.obs_hi, dims[0], &on->obs}, {"act", w.act_lo, w.act_hi, dims[1], &on->act},
+      {"state", w.state_lo, w.state_hi, dims[0], &on->state}};
   for (const auto& s : sets)
     for (int d = 0; d < s.n; ++d) {
       if (!(std::isfinite(s.lo[d]) && std::isfinite(s.hi[d]) && s.lo[d] <= s.hi[d])) {
@@ -647,19 +646,14 @@ static int make_dist(int env_id, const msacl_region_disturbance_t* w, RDist* r) 
                   (double)s.hi[d]);
         return MSACL_ERR_BAD_ARG;
       }
-      s.rlo[d] = s.lo[d];
-      s.rhi[d] = s.hi[d];
       if (s.lo[d] != 0.f || s.hi[d] != 0.f) *s.on = 1;
     }
   return MSACL_OK;
 }
 
-static int region_eval(const msacl_region_params_t* p, const msacl_region_disturbance_t* w, const float* image, int64_t n,
-                       const int64_t* n_dev, const float* lo, const float* hi, const msacl_region_out_t* out, void* stream) {
-  int D;
-  if (int rc = check_params(p, &D)) return rc;
-  RDist dist;
-  if (int rc = make_dist(p->env_id, w, &dist)) return rc;
+// msacl_region_eval after check_params
+static int region_eval(const msacl_region_params_t* p, const RDist& on, const float* image, int64_t n, const int64_t* n_dev,
+                       const float* lo, const float* hi, const msacl_region_out_t* out, void* stream) {
   if (n < 0 || !image || !lo || !hi || !out || !out->v_lo || !out->v_hi || !out->vm_lo || !out->vm_hi || !out->img_lo ||
       !out->img_hi || !out->flags || !out->margin) {
     set_error("region_eval: bad argument");
@@ -667,39 +661,8 @@ static int region_eval(const msacl_region_params_t* p, const msacl_region_distur
   }
   if ((reinterpret_cast<uintptr_t>(image) & 15) != 0) { set_error("region_eval: image must be 16-byte aligned"); return MSACL_ERR_BAD_ARG; }
   if (n == 0) return MSACL_OK;
-  MSACL_DISPATCH_ENV(p->env_id, { return eval_launch<ID>(p, dist, image, n, n_dev, lo, hi, out, (cudaStream_t)stream); });
+  MSACL_DISPATCH_ENV(p->env_id, { return eval_launch<ID>(p, on, image, n, n_dev, lo, hi, out, (cudaStream_t)stream); });
   return MSACL_OK;
-}
-
-static int region_round(const msacl_region_params_t* p, const msacl_region_bnb_t* b, const msacl_region_disturbance_t* w,
-                        const float* image, uint32_t* stack, int64_t top, int64_t k, const msacl_region_ws_t* ws, int64_t* stats,
-                        float* examples, int64_t* children, void* stream) {
-  int D;
-  if (int rc = check_params(p, &D)) return rc;
-  RDist dist;
-  if (int rc = make_dist(p->env_id, w, &dist)) return rc;
-  if (!b || b->max_depth < 1 || b->max_depth > MSACL_REGION_MAX_DEPTH || b->inner_level < 0 || b->inner_level > 31 ||
-      b->max_examples < 0 || !image || !stack || !ws || !stats || !children || k < 1 || top < k ||
-      (b->max_examples > 0 && !examples)) {
-    set_error("region_round: bad argument (need 1 <= max_depth <= %d, 1 <= k <= top)", (int)MSACL_REGION_MAX_DEPTH);
-    return MSACL_ERR_BAD_ARG;
-  }
-  cudaStream_t s = (cudaStream_t)stream;
-  const int64_t nb = (k + RB - 1) / RB;
-  uint32_t* cells = stack + (top - k) * (1 + D);
-  region_cells_kernel<<<(unsigned)nb, RB, 0, s>>>(*p, D, cells, k, *ws);
-  if (int rc = region_eval(p, w, image, k, nullptr, ws->lo, ws->hi, &ws->res, stream)) return rc;
-  region_probe_kernel<<<(unsigned)nb, RB, 0, s>>>(*p, *b, D, k, *ws, 0);
-  region_scan_kernel<<<1, RB, 0, s>>>(ws->scan, nb, ws->scan + 3 * nb);
-  region_probe_kernel<<<(unsigned)nb, RB, 0, s>>>(*p, *b, D, k, *ws, 1);
-  if (int rc = region_eval(p, w, image, k, ws->scan + 3 * nb, ws->plo, ws->phi, &ws->pres, stream)) return rc;
-  region_decide_kernel<<<(unsigned)nb, RB, 0, s>>>(*b, D, k, *ws, stats);
-  region_scan_kernel<<<1, RB, 0, s>>>(ws->scan + nb, nb, ws->scan + 3 * nb + 1);
-  region_scan_kernel<<<1, RB, 0, s>>>(ws->scan + 2 * nb, nb, ws->scan + 3 * nb + 2);
-  region_scatter_kernel<<<(unsigned)nb, RB, 0, s>>>(*b, D, k, *ws, cells, stats, examples);
-  if (cudaMemcpyAsync(children, ws->scan + 3 * nb + 1, sizeof(int64_t), cudaMemcpyDeviceToDevice, s) != cudaSuccess)
-    return check_launch("region_round");
-  return check_launch("region_round");
 }
 
 }  // namespace msacl
@@ -729,26 +692,40 @@ int msacl_region_pack(const msacl_region_nets_t* s, float* image, void* stream) 
 
 int msacl_region_eval(const msacl_region_params_t* p, const float* image, int64_t n, const int64_t* n_dev, const float* lo,
                       const float* hi, const msacl_region_out_t* out, void* stream) {
-  return region_eval(p, nullptr, image, n, n_dev, lo, hi, out, stream);
+  int D;
+  RDist on;
+  if (int rc = check_params(p, &D, &on)) return rc;
+  return region_eval(p, on, image, n, n_dev, lo, hi, out, stream);
 }
 
 int msacl_region_round(const msacl_region_params_t* p, const msacl_region_bnb_t* b, const float* image, uint32_t* stack,
                        int64_t top, int64_t k, const msacl_region_ws_t* ws, int64_t* stats, float* examples, int64_t* children,
                        void* stream) {
-  return region_round(p, b, nullptr, image, stack, top, k, ws, stats, examples, children, stream);
-}
-
-int msacl_region_eval_robust(const msacl_region_params_t* p, const float* image, int64_t n, const int64_t* n_dev, const float* lo,
-                             const float* hi, const msacl_region_out_t* out, void* stream, const msacl_region_disturbance_t* w) {
-  if (!w) { set_error("region_eval_robust: null disturbance"); return MSACL_ERR_BAD_ARG; }
-  return region_eval(p, w, image, n, n_dev, lo, hi, out, stream);
-}
-
-int msacl_region_round_robust(const msacl_region_params_t* p, const msacl_region_bnb_t* b, const float* image, uint32_t* stack,
-                              int64_t top, int64_t k, const msacl_region_ws_t* ws, int64_t* stats, float* examples,
-                              int64_t* children, void* stream, const msacl_region_disturbance_t* w) {
-  if (!w) { set_error("region_round_robust: null disturbance"); return MSACL_ERR_BAD_ARG; }
-  return region_round(p, b, w, image, stack, top, k, ws, stats, examples, children, stream);
+  int D;
+  RDist on;
+  if (int rc = check_params(p, &D, &on)) return rc;
+  if (!b || b->max_depth < 1 || b->max_depth > MSACL_REGION_MAX_DEPTH || b->inner_level < 0 || b->inner_level > 31 ||
+      b->max_examples < 0 || !image || !stack || !ws || !stats || !children || k < 1 || top < k ||
+      (b->max_examples > 0 && !examples)) {
+    set_error("region_round: bad argument (need 1 <= max_depth <= %d, 1 <= k <= top)", (int)MSACL_REGION_MAX_DEPTH);
+    return MSACL_ERR_BAD_ARG;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t nb = (k + RB - 1) / RB;
+  uint32_t* cells = stack + (top - k) * (1 + D);
+  region_cells_kernel<<<(unsigned)nb, RB, 0, s>>>(*p, D, cells, k, *ws);
+  if (int rc = region_eval(p, on, image, k, nullptr, ws->lo, ws->hi, &ws->res, stream)) return rc;
+  region_probe_kernel<<<(unsigned)nb, RB, 0, s>>>(*p, *b, D, k, *ws, 0);
+  region_scan_kernel<<<1, RB, 0, s>>>(ws->scan, nb, ws->scan + 3 * nb);
+  region_probe_kernel<<<(unsigned)nb, RB, 0, s>>>(*p, *b, D, k, *ws, 1);
+  if (int rc = region_eval(p, on, image, k, ws->scan + 3 * nb, ws->plo, ws->phi, &ws->pres, stream)) return rc;
+  region_decide_kernel<<<(unsigned)nb, RB, 0, s>>>(*b, D, k, *ws, stats);
+  region_scan_kernel<<<1, RB, 0, s>>>(ws->scan + nb, nb, ws->scan + 3 * nb + 1);
+  region_scan_kernel<<<1, RB, 0, s>>>(ws->scan + 2 * nb, nb, ws->scan + 3 * nb + 2);
+  region_scatter_kernel<<<(unsigned)nb, RB, 0, s>>>(*b, D, k, *ws, cells, stats, examples);
+  if (cudaMemcpyAsync(children, ws->scan + 3 * nb + 1, sizeof(int64_t), cudaMemcpyDeviceToDevice, s) != cudaSuccess)
+    return check_launch("region_round");
+  return check_launch("region_round");
 }
 
 }  // extern "C"

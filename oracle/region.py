@@ -98,13 +98,20 @@ def lyapunov(layers, x, tanh_act=True, xp=np):
     return (z * z).sum(-1)
 
 
-def closed_loop(name, policy_layers, x, steps, xp=np):
-    """[(mu, a, F^j(x)) for j = 1..steps] of the greedy closed loop."""
+def closed_loop(name, policy_layers, x, steps, xp=np, dist=None):
+    """[(mu, a, F^j(x)) for j = 1..steps] of the greedy closed loop, disturbed as
+    F_d(x) = Phi(x, clip(half tanh(mu(x + n)) + mid) + u) + w.  dist is None (no disturbance) or one (n, u, w) per step
+    ([N, D], [N, A], [N, D] arrays, any of them None for {0})."""
     A = SPECS[name].act_dim
     out = []
-    for _ in range(steps):
-        mu = policy_mean(policy_layers, x, A, xp)
+    for j in range(steps):
+        n, u, w = dist[j] if dist is not None else (None, None, None)
+        mu = policy_mean(policy_layers, x if n is None else x + n, A, xp)
         a = action(name, mu, xp)
+        if u is not None:
+            a = a + u
         x = env_step(name, x, a, xp)
+        if w is not None:
+            x = x + w
         out.append((mu, a, x))
     return out

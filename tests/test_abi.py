@@ -17,14 +17,14 @@ def header_symbols():
     return sorted(set(re.findall(r"\b(msacl_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_library_loads_and_exports_every_declared_symbol():
+def test_library_loads_and_exports_every_declared_symbol_at_abi_3():
     lib = msacl_b200.load_library()
     syms = header_symbols()
     assert len(syms) >= 15
     for s in syms:
         assert hasattr(lib, s), f"{s} declared in include/msacl_b200.h but not exported"
     assert sorted(_lib.SIGNATURES) == syms, "ctypes SIGNATURES and the header disagree"
-    assert lib.msacl_abi_version() == 2
+    assert lib.msacl_abi_version() == 3
 
 
 def test_env_dims_match_spec_table():

@@ -1,6 +1,6 @@
 """Region verifier under bounded disturbances, without a GPU: argument refusals and broadcasting of the disturbance boxes, the
-nominal report unchanged, robustness_margin's bracketing against a stubbed run, and the disturbed float64 closed loop that
-the GPU tests compare against."""
+nominal report unchanged, robustness_margin's bracketing against a stubbed run, and the disturbed float64 closed loop of the
+oracle that the GPU tests compare against."""
 import math
 
 import numpy as np
@@ -9,25 +9,6 @@ import pytest
 from oracle import envs as oenv
 from oracle import region as oreg
 from test_certify_region_cpu import BASE, _cells_to_stats, _make
-
-
-def closed_loop_disturbed(name, policy_layers, x, steps, dist=None, xp=np):
-    """[(mu, a, F^j(x)) for j = 1..steps] of the disturbed greedy closed loop
-    F_d(x) = Phi(x, clip(half tanh(mu(x + n)) + mid) + u) + w, built from the float64 oracle's unchanged pieces.  dist is
-    None or one (n, u, w) per step ([N, D], [N, A], [N, D] arrays, any of them None for {0})."""
-    A = oenv.SPECS[name].act_dim
-    out = []
-    for j in range(steps):
-        n, u, w = dist[j] if dist is not None else (None, None, None)
-        mu = oreg.policy_mean(policy_layers, x if n is None else x + n, A, xp)
-        a = oreg.action(name, mu, xp)
-        if u is not None:
-            a = a + u
-        x = oreg.env_step(name, x, a, xp)
-        if w is not None:
-            x = x + w
-        out.append((mu, a, x))
-    return out
 
 
 @pytest.mark.parametrize("dist,msg", [
@@ -46,6 +27,26 @@ def closed_loop_disturbed(name, policy_layers, x, steps, dist=None, xp=np):
 def test_disturbance_refusals(dist, msg):
     with pytest.raises(ValueError, match=msg):
         _make(disturbance=dist)
+
+
+def test_c_abi_refuses_bad_disturbance_bounds():
+    """msacl_region_eval / msacl_region_round check p->dist on the host before any launch: a non-finite bound or lo > hi in
+    the first obs_dim / act_dim entries is refused, naming the set and index; the entries after them are not read."""
+    import ctypes as C
+    from msacl_b200 import _lib
+    lib = _lib.load()
+    v = _make(env_name="DuctedFan", box=(-1.0, 1.0))
+    for key, j, lo, hi in [("obs", 5, 0.0, math.nan), ("act", 1, 0.2, 0.1), ("state", 0, -math.inf, 0.0)]:
+        p = v.params()
+        getattr(p.dist, key + "_lo")[j], getattr(p.dist, key + "_hi")[j] = lo, hi
+        assert lib.msacl_region_eval(C.byref(p), None, 0, None, None, None, None, None) == -2
+        assert f"disturbance {key}[{j}]".encode() in lib.msacl_last_error()
+        assert lib.msacl_region_round(C.byref(p), None, None, None, 1, 1, None, None, None, None, None) == -2
+        assert f"disturbance {key}[{j}]".encode() in lib.msacl_last_error()
+    p = v.params()
+    p.dist.obs_lo[6] = p.dist.state_hi[15] = math.nan
+    assert lib.msacl_region_eval(C.byref(p), None, 0, None, None, None, None, None) == -2
+    assert b"region_eval: bad argument" in lib.msacl_last_error()
 
 
 def test_disturbance_broadcasting_and_outward_rounding():
@@ -176,15 +177,20 @@ def test_disturbed_loop_with_zero_disturbance_is_the_nominal_loop(name):
     layers = [(W.astype(np.float64), b.astype(np.float64)) for W, b in w]
     rng = np.random.default_rng(2)
     x = rng.uniform(spec.obs_low * 0.1, spec.obs_high * 0.1, (256, D))
+    want, xj = [], x                     # the nominal loop, composed from its pieces
+    for _ in range(3):
+        mu = oreg.policy_mean(layers, xj, A)
+        a = oreg.action(name, mu)
+        xj = oreg.env_step(name, xj, a)
+        want.append((mu, a, xj))
     zero = [(np.zeros((256, D)), np.zeros((256, A)), np.zeros((256, D)))] * 3
-    want = oreg.closed_loop(name, layers, x, 3)
     for dist in (None, zero):
-        got = closed_loop_disturbed(name, layers, x, 3, dist)
+        got = oreg.closed_loop(name, layers, x, 3, dist=dist)
         for (m0, a0, x0), (m1, a1, x1) in zip(want, got):
             assert np.array_equal(m0, m1) and np.array_equal(a0, a1) and np.array_equal(x0, x1)
     # a nonzero process disturbance shifts the state after the step, an actuator one the action, sensor noise the policy input
     n, u, wd = rng.normal(size=(256, D)) * 1e-3, rng.normal(size=(256, A)) * 1e-3, rng.normal(size=(256, D)) * 1e-3
-    ((mu, a, x1),) = closed_loop_disturbed(name, layers, x, 1, [(n, u, wd)])
+    ((mu, a, x1),) = oreg.closed_loop(name, layers, x, 1, dist=[(n, u, wd)])
     assert np.array_equal(mu, oreg.policy_mean(layers, x + n, A))
     assert np.array_equal(a, oreg.action(name, mu) + u)
     assert np.array_equal(x1, oreg.env_step(name, x, a) + wd)

@@ -1,6 +1,6 @@
-"""Region verifier under bounded disturbances on the GPU: with zero disturbances the robust entry points are the nominal
-verifier bit for bit; enclosure of every layer against the float64 disturbed closed loop at corner and interior disturbance
-sequences; soundness of verified cells and of counterexamples under disturbances; robustness_margin; chunking invariance."""
+"""Region verifier under bounded disturbances on the GPU: explicit zero disturbances give the nominal verifier bit for bit;
+enclosure of every layer against the float64 disturbed closed loop at corner and interior disturbance sequences; soundness
+of verified cells and of counterexamples under disturbances; robustness_margin; chunking invariance."""
 import dataclasses
 
 import numpy as np
@@ -9,7 +9,6 @@ import torch
 
 from oracle import envs as oenv
 from oracle import region as oreg
-from test_certify_region_robust_cpu import closed_loop_disturbed
 from test_gpu_certify_region import BOX, RIN, TOL, _analytic_run, _analytic_vanderpol, _box, _inside, _layers, _networks
 
 pytestmark = pytest.mark.gpu
@@ -116,7 +115,7 @@ def test_enclosure_under_disturbances(name, m):
         seq = [tuple(_draw(ver.disturbance[k], N, p if j == 0 else (p + j) % P, g) for k in ("obs", "act", "state"))
                for j in range(m)]
         bump("V(x)", _inside(oreg.lyapunov(pv, x, tanh, torch), o["v_lo"], o["v_hi"]))
-        steps = closed_loop_disturbed(name, pl, x, m, seq, torch)
+        steps = oreg.closed_loop(name, pl, x, m, torch, dist=seq)
         for j, (mu, a, xj) in enumerate(steps):
             t = tr[:, j]
             bump("mu", _inside(mu, t[:, :A], t[:, A:2 * A]))
@@ -150,7 +149,7 @@ def test_analytic_vanderpol_small_process_disturbance():
         x = lo + (hi - lo) * torch.rand(lo.shape, device="cuda", generator=g, dtype=torch.float64)
         w = _draw(wbox, x.shape[0], p % 16, g)
         v0 = oreg.lyapunov(pv, x, True, torch)
-        x1 = closed_loop_disturbed("VanderPol", pl, x, 1, [(None, None, w)], torch)[-1][2]
+        x1 = oreg.closed_loop("VanderPol", pl, x, 1, torch, dist=[(None, None, w)])[-1][2]
         v1 = oreg.lyapunov(pv, x1, True, torch)
         bad += int((v1 > (1 - eta) * v0 * (1 + TOL)).sum()) + int((x1.abs() >= 10.0).any(-1).sum())
         total += x.shape[0]
@@ -174,7 +173,7 @@ def test_large_constant_bias_is_refuted_with_sound_margins():
     v0 = oreg.lyapunov(pv, x, True, torch)
     for p in range(64):                                   # the corners (p < 8 of _draw) and random interior draws
         u, w = _draw(boxes["act"], x.shape[0], p, g), _draw(boxes["state"], x.shape[0], p, g)
-        x1 = closed_loop_disturbed("VanderPol", pl, x, 1, [(None, u, w)], torch)[-1][2]
+        x1 = oreg.closed_loop("VanderPol", pl, x, 1, torch, dist=[(None, u, w)])[-1][2]
         viol = torch.where(dec, oreg.lyapunov(pv, x1, True, torch) - (1 - eta) * v0, (x1.abs() - 10.0).max(-1).values)
         assert bool((viol >= marg * (1 - 1e-9)).all()), (p, float((viol - marg).min()))
 
