@@ -287,3 +287,175 @@ def test_fused_learner_matches_torch_engine(env, B, sizes):
     sa, sb = a.networks.state_dict(), b.networks.state_dict()
     for k in sa:
         assert float((sa[k] - sb[k]).abs().max()) <= 4e-3, k
+
+
+def _lib_st():
+    import msacl_b200
+    from msacl_b200 import _lib
+    return msacl_b200.load_library(), _lib, _lib.current_stream()
+
+
+@pytest.mark.parametrize("A", [1, 2, 8])
+def test_policy_logits_grad_edges_vs_torch_autograd(A):
+    """msacl_policy_logits_grad (critic path + entropy term + clipped surrogate on step 0 of each window) vs torch float32
+    autograd of the same loss, at its edges: log_std exactly at min_log_std / max_log_std and beyond them (the clamp passes
+    the gradient at the bounds), stored actions exactly at the action bounds (replay actions are clipped; the atanh argument
+    is computed as the reference computes it, in float32), |u| > 9 where tanh is +-1 in float32, A = 1 and A = 8 (LA_MAX),
+    and step-0 ratios on both sides of 1 - clip and 1 + clip."""
+    from msacl_b200.algorithm import TanhGauss
+    lib, _lib, st = _lib_st()
+    g = torch.Generator(device="cuda").manual_seed(A)
+    B, n, D, clip, min_ls, max_ls = 96, 4, 3, 0.1, -2.0, 0.5
+    M = B * n
+    r = lambda *s: torch.randn(*s, device="cuda", generator=g)
+    lo = torch.tensor([-2.0, 0.0, -1.0, -5.0, -0.5, -3.0, 0.0, -1.0][:A], device="cuda")
+    hi = torch.tensor([2.0, 3.0, 5.0, 5.0, 0.5, 1.0, 85.064, 1.0][:A], device="cuda")
+    mean, ls = 0.5 * r(M, A), min_ls + (max_ls - min_ls) * torch.rand(M, A, device="cuda", generator=g)
+    kind = torch.arange(M, device="cuda") % 8
+    ls = torch.where(kind[:, None] == 1, torch.full_like(ls, min_ls), ls)        # exactly at the bounds ...
+    ls = torch.where(kind[:, None] == 2, torch.full_like(ls, max_ls), ls)
+    ls = torch.where(kind[:, None] == 3, min_ls - 0.5 - torch.rand_like(ls), ls)  # ... and beyond them
+    ls = torch.where(kind[:, None] == 4, max_ls + 0.5 + torch.rand_like(ls), ls)
+    eps = r(M, A)
+    eps = torch.where(kind[:, None] == 5, torch.where(eps >= 0, 12.0, -12.0), eps)    # |u| > 9: tanh(u) = +-1 in float32
+    mid, half = (hi + lo) / 2, (hi - lo) / 2
+    act = mid + half * (1.9 * torch.rand(M, A, device="cuda", generator=g) - 0.95)
+    at_bound = (kind == 6) | (kind == 7)
+    act = torch.where(at_bound[:, None], torch.where(r(M, A) > 0, hi, lo), act)       # stored actions on the bounds
+    logits = torch.cat([mean, ls], 1).contiguous()
+    dxq1, dxq2 = r(M, D + A) / M, r(M, D + A) / M
+    la = torch.tensor([-0.4], device="cuda")
+    adv = r(B)
+
+    def dist_of(lg):
+        return TanhGauss(torch.cat([lg[:, :A], torch.clamp(lg[:, A:], min_ls, max_ls).exp()], 1), lo, hi)
+
+    with torch.no_grad():
+        lp0 = dist_of(logits).log_prob(act)
+    log_ratio = torch.tensor([-0.5, -0.2, -0.05, 0.05, 0.2, 0.5], device="cuda")[torch.arange(M, device="cuda") % 6]
+    old_logp = (lp0 - log_ratio).contiguous()
+    first = torch.arange(M, device="cuda") % n == 0
+    # torch float32 reference of the loss whose logits gradient the kernel writes
+    lg = logits.clone().requires_grad_(True)
+    dist = dist_of(lg)
+    new_act, new_logp = dist.rsample(eps)
+    ratio = torch.exp(dist.log_prob(act)[first] - old_logp[first])
+    surr = torch.min(ratio * adv, torch.clamp(ratio, 1 - clip, 1 + clip) * adv)
+    loss = (new_act * (dxq1 + dxq2)[:, D:]).sum() + la.exp() * new_logp.mean() - surr.mean()
+    loss.backward()
+    got = torch.full((M, 2 * A), float("nan"), device="cuda")
+    sums = torch.zeros(3, dtype=torch.float64, device="cuda")
+    _lib.check(lib.msacl_policy_logits_grad(M, n, D, A, logits.data_ptr(), eps.contiguous().data_ptr(), dxq1.data_ptr(), dxq2.data_ptr(),
+                                            la.data_ptr(), act.contiguous().data_ptr(), old_logp.data_ptr(), adv.data_ptr(), clip,
+                                            lo.data_ptr(), hi.data_ptr(), min_ls, max_ls, got.data_ptr(), sums.data_ptr(), st))
+    want = lg.grad
+    scale = float(want.abs().max())
+    err = (got - want).abs() / scale
+    print(f"A={A}: max err / max|g| {float(err.max()):.2e}, rows with actions on the bounds {float(err[at_bound].max()):.2e}")
+    np.testing.assert_allclose(got.cpu().numpy(), want.cpu().numpy(), rtol=2e-4, atol=2e-5 * scale)
+    # the kernel's ratios come from its own log_prob (float32, round-off apart): 1e-5 of the sum of |min(surr1, surr2)|
+    assert abs(float(sums[2]) - float(surr.double().sum())) <= 1e-5 * float(surr.double().abs().sum())
+    # every edge is exercised: clamped log_std columns get no gradient, the bound values do
+    assert (got[kind == 3][:, A:] == 0).all() and (got[kind == 4][:, A:] == 0).all()
+    assert (got[(kind == 1) | (kind == 2)][:, A:] != 0).all()
+    r0 = ratio.detach()
+    assert ((r0 < 1 - clip) & (adv > 0)).any() and ((r0 < 1 - clip) & (adv < 0)).any()
+    assert ((r0 > 1 + clip) & (adv > 0)).any() and ((r0 > 1 + clip) & (adv < 0)).any() and ((r0 > 1 - clip) & (r0 < 1 + clip)).any()
+
+
+def test_policy_q_route_exact_ties_vs_torch_minimum():
+    """msacl_policy_q_route vs torch autograd of -mean(torch.minimum(q1, q2) - alpha logp): half the gradient to each critic
+    on an exact tie; the two double-atomic sums vs float64."""
+    lib, _lib, st = _lib_st()
+    g = torch.Generator(device="cuda").manual_seed(4)
+    rows = 3000
+    q1 = torch.randn(rows, device="cuda", generator=g)
+    q2 = torch.where(torch.arange(rows, device="cuda") % 3 == 0, q1, torch.randn(rows, device="cuda", generator=g))
+    lp = torch.randn(rows, device="cuda", generator=g) - 2.0
+    la = torch.tensor([0.3], device="cuda")
+    a, b = q1.clone().requires_grad_(True), q2.clone().requires_grad_(True)
+    (-(torch.minimum(a, b) - la.exp() * lp).mean()).backward()
+    dq1, dq2 = torch.empty(rows, device="cuda"), torch.empty(rows, device="cuda")
+    sums = torch.full((3,), 7.0, dtype=torch.float64, device="cuda")
+    _lib.check(lib.msacl_policy_q_route(rows, q1.data_ptr(), q2.data_ptr(), lp.data_ptr(), la.data_ptr(), dq1.data_ptr(), dq2.data_ptr(),
+                                        sums.data_ptr(), st))
+    assert int((q1 == q2).sum()) == 1000
+    np.testing.assert_allclose(dq1.cpu().numpy(), a.grad.cpu().numpy(), rtol=1e-6, atol=0)
+    np.testing.assert_allclose(dq2.cpu().numpy(), b.grad.cpu().numpy(), rtol=1e-6, atol=0)
+    alpha = float(torch.tensor(0.3).exp())
+    np.testing.assert_allclose(float(sums[0]), float((torch.minimum(q1, q2).double() - alpha * lp.double()).sum()), rtol=1e-5)
+    np.testing.assert_allclose(float(sums[1]), float(lp.double().sum()), rtol=1e-6)
+    assert float(sums[2]) == 0.0
+
+
+def test_q_backup_and_loss_grad_grid_stride_vs_float64():
+    """msacl_q_backup_dev_alpha and msacl_q_loss_grad over more rows than one pass of the grid (148 * 8 * 256), so every
+    thread strides; dq = 2 (q - y) / count and the four double-atomic sums vs float64."""
+    lib, _lib, st = _lib_st()
+    g = torch.Generator(device="cuda").manual_seed(9)
+    count = 2 * 148 * 8 * 256 + 77
+    r = lambda: torch.randn(count, device="cuda", generator=g)
+    rew, nq1, nq2, nlp, q1, q2 = -torch.rand(count, device="cuda", generator=g) * 5, r(), r(), r() - 1, r(), r()
+    done = (torch.rand(count, device="cuda", generator=g) < 0.2).float()
+    la = torch.tensor([-0.25], device="cuda")
+    backup = torch.empty(count, device="cuda")
+    _lib.check(lib.msacl_q_backup_dev_alpha(count, rew.data_ptr(), done.data_ptr(), nq1.data_ptr(), nq2.data_ptr(), nlp.data_ptr(), 0.99,
+                                            la.data_ptr(), backup.data_ptr(), st))
+    alpha = float(np.exp(np.float32(-0.25)))
+    want = rew.double() + (1 - done.double()) * 0.99 * (torch.minimum(nq1, nq2).double() - alpha * nlp.double())
+    assert float((backup.double() - want).abs().max()) <= 2e-6 * float(want.abs().max())
+    dq1, dq2 = torch.full_like(q1, float("nan")), torch.full_like(q2, float("nan"))
+    sums = torch.full((4,), 7.0, dtype=torch.float64, device="cuda")
+    _lib.check(lib.msacl_q_loss_grad(count, q1.data_ptr(), q2.data_ptr(), backup.data_ptr(), dq1.data_ptr(), dq2.data_ptr(), sums.data_ptr(), st))
+    y = backup.double()
+    for got, q in ((dq1, q1), (dq2, q2)):
+        np.testing.assert_allclose(got.cpu().numpy(), (2 * (q.double() - y) / count).cpu().numpy(), rtol=1e-6, atol=0)
+    want = [((q1.double() - y) ** 2).sum(), ((q2.double() - y) ** 2).sum(), q1.double().sum(), q2.double().sum()]
+    scale = [want[0], want[1], q1.double().abs().sum(), q2.double().abs().sum()]
+    for i in range(4):
+        assert abs(float(sums[i] - want[i])) <= 1e-6 * float(scale[i]), (i, float(sums[i]), float(want[i]))
+
+
+@pytest.mark.parametrize("cols", [32, 256])
+def test_sumsq_bwd_vs_float64(cols):
+    """msacl_sumsq_bwd: dz = 2 z dV for V = sum_j z_j^2 (the Lyapunov head), at 32 and 256 output columns."""
+    lib, _lib, st = _lib_st()
+    g = torch.Generator(device="cuda").manual_seed(cols)
+    rows = 1234
+    z, dv = torch.randn(rows, cols, device="cuda", generator=g), torch.randn(rows, device="cuda", generator=g)
+    dz = torch.full_like(z, float("nan"))
+    _lib.check(lib.msacl_sumsq_bwd(rows, cols, z.data_ptr(), dv.data_ptr(), dz.data_ptr(), st))
+    zz = z.double().clone().requires_grad_(True)
+    ((zz ** 2).sum(1) * dv.double()).sum().backward()
+    np.testing.assert_allclose(dz.cpu().numpy(), zz.grad.cpu().numpy(), rtol=1e-7, atol=0)
+
+
+@pytest.mark.parametrize("alpha_bound", [None, 0.72])
+def test_alpha_update_steps_match_torch_adam(alpha_bound):
+    """msacl_adam_tick + msacl_alpha_update, several steps, vs torch.optim.Adam on a float32 log_alpha with
+    loss_alpha = exp(log_alpha) (entropy - target), with and without the alpha_bound clamp after the step."""
+    import math
+    lib, _lib, st = _lib_st()
+    rows, target, lr = 1024, -2.0, 1e-2
+    p = torch.nn.Parameter(torch.tensor(math.log(0.7)))
+    opt = torch.optim.Adam([p], lr=lr)
+    la = torch.tensor([math.log(0.7)], device="cuda")
+    step, dyn = torch.zeros(1, dtype=torch.int32, device="cuda"), torch.zeros(2, device="cuda")
+    state, ent_out = torch.zeros(2, device="cuda"), torch.zeros(1, device="cuda")
+    clamp = math.log(alpha_bound) if alpha_bound else float("inf")
+    for k, entropy in enumerate([-3.0, -2.5, -4.0, -2.25, -3.5, -1.5]):      # entropy below the target: log_alpha grows
+        sums = torch.tensor([0.0, -entropy * rows, 0.0], dtype=torch.float64, device="cuda")
+        _lib.check(lib.msacl_adam_tick(step.data_ptr(), dyn.data_ptr(), lr, 0.9, 0.999, st))
+        _lib.check(lib.msacl_alpha_update(la.data_ptr(), sums.data_ptr(), rows, target, state.data_ptr(), 0.1, 0.999, 0.001, 0.0, 1.0, 1e-8,
+                                          clamp, ent_out.data_ptr(), dyn.data_ptr(), st))
+        opt.zero_grad()
+        (p.exp() * (torch.tensor(entropy) - target)).backward()
+        opt.step()
+        if alpha_bound:
+            with torch.no_grad():
+                p.clamp_(max=math.log(alpha_bound))
+        assert float(ent_out) == entropy
+        np.testing.assert_allclose(float(la), float(p), rtol=2e-6, atol=1e-7, err_msg=f"step {k + 1}")
+    assert int(step) == 6
+    if alpha_bound:
+        assert float(la) == float(np.float32(math.log(alpha_bound)))
